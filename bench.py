@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200-native BlueSky-Gym step path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 Workload at every N (weak scaling): BASELINE.json configs[1] per GPU -- HorizontalCREnv-v0, 4096 env
 instances, 20 intruders each (21 aircraft), StateBased conflict detection in every simulator substep,
@@ -11,6 +11,8 @@ Metric: env-steps/s, whole job.  Extra: CD aircraft-pairs/s at N = 100k (BASELIN
 
 Prints ONE JSON line (rank 0).  `--impl reference` times the CPU restatement of the reference's step
 loop (oracle/, "port": the reference's own BlueSky dependency is not installable here) on the host cores.
+`--dump-outputs DIR` writes what the last timed step returned on rank 0 (obs keys, reward, terminated, truncated of
+every env, float32) as DIR/<name>.npy: the inputs depend only on the arguments, so two builds can be compared.
 """
 import argparse
 import json
@@ -148,7 +150,7 @@ def run_reference(args):
     cores = os.cpu_count() or 1
     why_not = probe_real_reference()
     real = why_not is None
-    K, W = max(1, args.steps), max(0, args.warmup)
+    K, W = args.steps, max(0, args.warmup)
     ctx = mp.get_context("spawn")
     with ctx.Pool(cores) as pool:
         try:
@@ -335,10 +337,11 @@ def run_b200(args):
         for i in range(K):
             flush.fill_(float(i))                           # evict the sim state from L2 (not timed)
             ev[i][0].record()
-            venv.step_torch(bank[W + i])
+            out = venv.step_torch(bank[W + i])
             ev[i][1].record()
         barrier()
     launches = venv.gpu_launches - launches0
+    dumped = step_outputs(*out) if args.dump_outputs and rank == 0 else None     # (the next step overwrites them)
     t_dev = sum(a.elapsed_time(b) for a, b in ev) * 1e-3
     t_dev = max_over_ranks(t_dev)
     value = E * world * K / t_dev
@@ -482,8 +485,20 @@ def run_b200(args):
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
+    if dumped is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     if line is not None:
         print(json.dumps(line), file=_OUT, flush=True)
+
+
+def step_outputs(obs, reward, terminated, truncated):
+    """Host float32 copies of what BlueSkyVectorEnv.step_torch returned, by --dump-outputs file name (E x 103 obs values
+    + 3 x E: 1.7 MB at 4096 envs)."""
+    arrays = {"obs_" + k: v for k, v in obs.items()}
+    arrays.update(reward=reward, terminated=terminated, truncated=truncated)
+    return {k: v.float().cpu().numpy() for k, v in arrays.items()}
 
 
 def bench_env_leg(torch, dev, BlueSkyVectorEnv, env_id, E, kw, world, rank, max_over_ranks, barrier, steps=60):
@@ -843,7 +858,12 @@ def main():
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--skip-cpu", action="store_true", help="omit the cpu_baseline leg (profiling runs under ncu)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 step path")
     # The contract is ONE JSON line on stdout.  Libraries write banners to fd 1 from native code (NCCL prints its version
     # there when NCCL_DEBUG asks for it), so fd 1 points at stderr while the bench runs and the line goes to the saved fd.
     global _OUT
