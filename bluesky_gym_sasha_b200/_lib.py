@@ -123,71 +123,57 @@ def load():
     lib.bsg_step.argtypes = [vp, vp, vp]
     lib.bsg_step_host.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp]
     lib.bsg_step_host_block.argtypes = [vp, vp, vp, C.c_size_t, vp]
-    if hasattr(lib, "bsg_step_host_begin"):     # (absent only in older A/B builds loaded through BSG_B200_LIB)
-        lib.bsg_step_host_begin.argtypes = [vp, vp, vp, C.c_size_t, vp]
-        lib.bsg_step_host_begin.restype = C.c_int
-        lib.bsg_step_host_wait.argtypes = [vp, vp, vp, C.c_size_t]
-        lib.bsg_step_host_wait.restype = C.c_int
+    lib.bsg_step_host_begin.argtypes = [vp, vp, vp, C.c_size_t, vp]
+    lib.bsg_step_host_begin.restype = C.c_int
+    lib.bsg_step_host_wait.argtypes = [vp, vp, vp, C.c_size_t]
+    lib.bsg_step_host_wait.restype = C.c_int
     lib.bsg_set_obs_noise.argtypes = [vp, f32]
     lib.bsg_set_obs_noise.restype = C.c_int
-    if hasattr(lib, "bsg_set_seed"):
-        lib.bsg_set_seed.argtypes = [vp, C.c_uint64]
-        lib.bsg_set_seed.restype = C.c_int
-    if hasattr(lib, "bsg_set_wind"):            # (absent only in older A/B builds loaded through BSG_B200_LIB)
-        lib.bsg_set_wind.argtypes = [vp, C.POINTER(Wind)]
-        lib.bsg_set_wind.restype = C.c_int
-    if hasattr(lib, "bsg_load_state"):          # (absent only in older A/B builds loaded through BSG_B200_LIB)
-        lib.bsg_load_state.argtypes = [vp, i32, C.POINTER(AcState), vp]
-        lib.bsg_load_state.restype = C.c_int
-        lib.bsg_get_noise_calls.argtypes = [vp, C.POINTER(u32)]
-        lib.bsg_get_noise_calls.restype = C.c_int
-        lib.bsg_set_noise_calls.argtypes = [vp, u32]
-        lib.bsg_set_noise_calls.restype = C.c_int
+    lib.bsg_set_seed.argtypes = [vp, C.c_uint64]
+    lib.bsg_set_seed.restype = C.c_int
+    lib.bsg_set_wind.argtypes = [vp, C.POINTER(Wind)]
+    lib.bsg_set_wind.restype = C.c_int
+    lib.bsg_load_state.argtypes = [vp, i32, C.POINTER(AcState), vp]
+    lib.bsg_load_state.restype = C.c_int
+    lib.bsg_get_noise_calls.argtypes = [vp, C.POINTER(u32)]
+    lib.bsg_get_noise_calls.restype = C.c_int
+    lib.bsg_set_noise_calls.argtypes = [vp, u32]
+    lib.bsg_set_noise_calls.restype = C.c_int
     lib.bsg_host_copy.argtypes = [vp, vp, C.c_size_t]
     lib.bsg_host_copy.restype = C.c_int
-    if hasattr(lib, "bsg_host_widen"):          # (absent only in older A/B builds loaded through BSG_B200_LIB)
-        lib.bsg_host_widen.argtypes = [vp, vp, C.c_size_t]
-        lib.bsg_host_widen.restype = C.c_int
+    lib.bsg_host_widen.argtypes = [vp, vp, C.c_size_t]
+    lib.bsg_host_widen.restype = C.c_int
     lib.bsg_step_host_copy.argtypes = [vp, vp, vp, C.c_size_t, vp, C.c_size_t, vp]
     lib.bsg_traf_update.argtypes = [vp, i32, vp]
-    if hasattr(lib, "bsg_render"):              # (absent only in older A/B builds loaded through BSG_B200_LIB)
-        lib.bsg_render.argtypes = [vp, i32, i32, i32, u32, vp, vp]
-        lib.bsg_render.restype = C.c_int
-    if hasattr(lib, "bsg_traf_substep"):        # (absent only in older A/B builds loaded through BSG_B200_LIB)
-        lib.bsg_traf_pack.argtypes = [C.POINTER(TrafConfig), C.POINTER(TrafTensors), vp, vp]
-        lib.bsg_traf_activate.argtypes = [C.POINTER(TrafConfig), C.POINTER(TrafTensors), vp]
-        lib.bsg_traf_substep.argtypes = [C.POINTER(TrafConfig), C.POINTER(TrafTensors), vp, i32, vp, vp, vp, vp, i64, vp, i64, vp]
-        lib.bsg_traf_workspace.argtypes = [i64, i64]
-        lib.bsg_traf_workspace.restype = i64
-        for f in (lib.bsg_traf_pack, lib.bsg_traf_activate, lib.bsg_traf_substep):
-            f.restype = C.c_int
+    lib.bsg_render.argtypes = [vp, i32, i32, i32, u32, vp, vp]
+    lib.bsg_render.restype = C.c_int
+    lib.bsg_traf_pack.argtypes = [C.POINTER(TrafConfig), C.POINTER(TrafTensors), vp, vp]
+    lib.bsg_traf_activate.argtypes = [C.POINTER(TrafConfig), C.POINTER(TrafTensors), vp]
+    lib.bsg_traf_substep.argtypes = [C.POINTER(TrafConfig), C.POINTER(TrafTensors), vp, i32, vp, vp, vp, vp, i64, vp, i64, vp]
+    lib.bsg_traf_workspace.argtypes = [i64, i64]
+    lib.bsg_traf_workspace.restype = i64
     lib.bsg_cd_padded.argtypes = [i64]
     lib.bsg_cd_padded.restype = i64
     lib.bsg_cd_pack.argtypes = [vp, vp, vp, vp, vp, vp, i64, f64, f64, vp, vp]
-    if hasattr(lib, "bsg_cd_pack_ordered"):     # (absent only in older A/B builds loaded through BSG_B200_LIB)
-        lib.bsg_cd_order_workspace.argtypes = [i64]
-        lib.bsg_cd_order_workspace.restype = i64
-        lib.bsg_cd_pack_ordered.argtypes = [vp, vp, vp, vp, vp, vp, i64, f64, f64, vp, vp, vp, i64, vp]
+    lib.bsg_cd_order_workspace.argtypes = [i64]
+    lib.bsg_cd_order_workspace.restype = i64
+    lib.bsg_cd_pack_ordered.argtypes = [vp, vp, vp, vp, vp, vp, i64, f64, f64, vp, vp, vp, i64, vp]
     lib.bsg_cd_detect.argtypes = [vp, i64, i64, i64, f32, f32, f32, u32, vp, vp, vp, vp, C.POINTER(CdLists), vp]
-    if hasattr(lib, "bsg_cd_detect_culled"):
-        lib.bsg_cd_cull_workspace.argtypes = [i64, i64]
-        lib.bsg_cd_cull_workspace.restype = i64
-        lib.bsg_cd_detect_culled.argtypes = [vp, i64, i64, i64, f32, f32, f32, u32, vp, vp, vp, vp, C.POINTER(CdLists), vp, i64, vp]
-        lib.bsg_cd_detect_culled.restype = C.c_int
-    if hasattr(lib, "bsg_cd_detect_peers"):
-        lib.bsg_cd_detect_peers.argtypes = [C.POINTER(vp), i32, i32, i64, f32, f32, f32, u32, vp, vp, vp, vp, C.POINTER(CdLists), vp, i64, vp]
-        lib.bsg_cd_detect_peers.restype = C.c_int
+    lib.bsg_cd_cull_workspace.argtypes = [i64, i64]
+    lib.bsg_cd_cull_workspace.restype = i64
+    lib.bsg_cd_detect_culled.argtypes = [vp, i64, i64, i64, f32, f32, f32, u32, vp, vp, vp, vp, C.POINTER(CdLists), vp, i64, vp]
+    lib.bsg_cd_detect_peers.argtypes = [C.POINTER(vp), i32, i32, i64, f32, f32, f32, u32, vp, vp, vp, vp, C.POINTER(CdLists), vp, i64, vp]
     lib.bsg_probe_fp32.argtypes = [i32, C.POINTER(f64)]
+    lib.bsg_abi_struct_size.argtypes = [C.c_int]
+    lib.bsg_abi_struct_size.restype = C.c_int
     for name in ("bsg_query_layout", "bsg_create", "bsg_bind_state", "bsg_reset", "bsg_step", "bsg_step_host", "bsg_step_host_block", "bsg_step_host_copy",
-                 "bsg_traf_update", "bsg_cd_pack", "bsg_cd_detect", "bsg_probe_fp32"):
+                 "bsg_traf_update", "bsg_traf_pack", "bsg_traf_activate", "bsg_traf_substep", "bsg_cd_pack", "bsg_cd_pack_ordered",
+                 "bsg_cd_detect", "bsg_cd_detect_culled", "bsg_cd_detect_peers", "bsg_probe_fp32"):
         getattr(lib, name).restype = C.c_int
-    if hasattr(lib, "bsg_abi_struct_size"):     # (absent only in older A/B builds loaded through BSG_B200_LIB)
-        lib.bsg_abi_struct_size.argtypes = [C.c_int]
-        lib.bsg_abi_struct_size.restype = C.c_int
-        for which, st in enumerate((Config, Layout, TensorTable, Wind, Perf, AcState, CdLists)):
-            if lib.bsg_abi_struct_size(which) != C.sizeof(st):
-                raise BsgError(f"{LIB_PATH}: sizeof({st.__name__}) is {lib.bsg_abi_struct_size(which)} in the library, "
-                               f"{C.sizeof(st)} in bluesky_gym_sasha_b200/_lib.py (include/bsg.h changed: rebuild / update the binding)")
+    for which, st in enumerate((Config, Layout, TensorTable, Wind, Perf, AcState, CdLists, TrafConfig, TrafTensors)):
+        if lib.bsg_abi_struct_size(which) != C.sizeof(st):
+            raise BsgError(f"{LIB_PATH}: sizeof({st.__name__}) is {lib.bsg_abi_struct_size(which)} in the library, "
+                           f"{C.sizeof(st)} in bluesky_gym_sasha_b200/_lib.py (include/bsg.h changed: rebuild / update the binding)")
     _lib = lib
     return lib
 

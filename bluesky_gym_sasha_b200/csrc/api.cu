@@ -414,10 +414,10 @@ extern "C" int bsg_step_host_copy(bsg_handle* h, const float* h_actions, void* h
     const char* d0 = (const char*)h->t.obs;
     char* h0 = (char*)h_block;
     if (dst) bsg::host_pool_prewake();     // the copy threads wake up while the GPU is busy
-    // chunks: small transfers go in one piece; otherwise 4 pieces of the copied region, the tail with the last
-    static const int want = [] { const char* e = getenv("BSG_D2H_CHUNKS"); int v = e ? atoi(e) : 2; return v < 1 ? 1 : (v > 4 ? 4 : v); }();
-    const int nchunk = (dst && dst_bytes >= (512u << 10)) ? want : 1;
-    size_t bounds[5];
+    // chunks: small transfers go in one piece; otherwise 2 pieces of the copied region, the tail with the last
+    // (1, 2 and 4 pieces measured equal once the copy threads are pre-woken: DESIGN §4)
+    const int nchunk = (dst && dst_bytes >= (512u << 10)) ? 2 : 1;
+    size_t bounds[3];
     for (int k = 0; k <= nchunk; ++k) bounds[k] = (dst_bytes * k / nchunk) & ~(size_t)255;
     bounds[0] = 0;
     bounds[nchunk] = nbytes;

@@ -352,11 +352,9 @@ __device__ __forceinline__ void cd_process_item(const CdArgs& a, float (*s_tile)
     }
 }
 
-#ifndef BSG_CD_MINBLOCKS
-#define BSG_CD_MINBLOCKS 4
-#endif
+// 4 CTAs per SM (124 registers); 5 (96 registers, no spills) measured slower (DESIGN §4)
 template <bool WRAP, bool LIST, bool SYM>
-__global__ void __launch_bounds__(kNT, BSG_CD_MINBLOCKS) cd_tiled_kernel(const CdArgs a) {
+__global__ void __launch_bounds__(kNT, 4) cd_tiled_kernel(const CdArgs a) {
     __shared__ __align__(128) float s_tile[2][kTileFloats];
     __shared__ __align__(8) uint64_t s_full[2];
     __shared__ int s_item[3];

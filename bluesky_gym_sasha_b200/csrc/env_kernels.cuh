@@ -24,11 +24,8 @@
 
 namespace bsg {
 
-#ifndef BSG_ENV_THREADS
-#define BSG_ENV_THREADS 128
-#endif
-constexpr int kEnvThreads = BSG_ENV_THREADS;
-constexpr int kEnvBlocksPerSm = 896 / BSG_ENV_THREADS;      // 28 warps per SM: what 72 registers per thread allow
+constexpr int kEnvThreads = 128;
+constexpr int kEnvBlocksPerSm = 7;      // 28 warps per SM: what 72 registers per thread allow
 constexpr uint32_t kFlAlive = 1u, kFlLnav = 2u, kFlLastWp = 4u, kFlTgt = 8u /* aux.w caches allow_tas */, kFlWpShift = 8u;
 enum { kModeStep = 0, kModeReset = 1, kModeTraf = 2 };
 
@@ -446,7 +443,7 @@ __device__ __forceinline__ void ac_kinematics(Ac& a, const EnvParams& P, const T
 //     (B) pairs among the other aircraft (a ring of m = n - 1 members; lane r tests the offsets 1 .. m/2, two per
 //         iteration in packed f32x2, records staged as a structure of arrays written twice, m apart, so that
 //         (r + k) mod m is a plain offset) are filtered when the env step starts and again only after one of them
-//         moved its ground-speed vector by more than kCdVelTol (BSG_CD_REUSE).  With w(t) = w0 + eps(t), |eps| <= dw,
+//         moved its ground-speed vector by more than kCdVelTol.  With w(t) = w0 + eps(t), |eps| <= dw,
 //         d x w and d . w - t |w0|^2 stay within dw (|d0| + 2 t |w0| + t dw) of their values at the filter pass, plus
 //         the flat-earth terms -- cos(mean lat) and the longitude rate drift as the pair moves in latitude -- which
 //         change dcpa by at most  kappa (|dx| + |dy| + d0),  kappa = 1.5 T vmax tan(lat_max) / Re,  d0 = (4 vmax + 1) T,
@@ -462,13 +459,6 @@ __device__ __forceinline__ void ac_kinematics(Ac& a, const EnvParams& P, const T
 // ====================================================================================================
 enum { HX = 0, HY = 1, HCH = 2, HSH = 3, HU = 4, HV = 5, kHotFields = 6 };
 constexpr int kQueuePerThread = 16;      // queue entries per lane: (B) <= (G-1)(G-2)/2 plus (A) <= G-1 < 16 G for G <= 32
-#ifndef BSG_HOT_UNROLL
-#define BSG_HOT_UNROLL 1
-#endif
-constexpr int kHotUnroll = BSG_HOT_UNROLL;
-#ifndef BSG_CD_REUSE
-#define BSG_CD_REUSE 1
-#endif
 constexpr float kCdVelTol = 0.15f;       // [m/s] |du| + |dv| an aircraft may drift from the velocity of the kept (B) pass
 constexpr float kCdAbsEps = 1.0f;        // [m^2/s] rounding slack of the |d x w|, d . w tests at |w| ~ 0
 
@@ -505,22 +495,12 @@ struct __align__(16) GroupSmem {
 // creep every substep) keeps a (B) list while every ring aircraft stays within kCdVelTol of the velocity the list was built
 // with; otherwise the list is rebuilt as soon as any ring aircraft moved at all (the intruders of HorizontalCR / SectorCR
 // never do).  Rebuilding more often never changes results: every list is a superset of what the exact phase accepts.
-#ifdef BSG_SUBSTEP_CLOCKS
-__device__ long long g_clk[16];
-#define BSG_CLK(k) do { if (clk_on) g_clk[k] = clock64(); } while (0)
-#else
-#define BSG_CLK(k) do { } while (0)
-#endif
 template <int G, bool TOL>
 __device__ __forceinline__ void group_cd(GroupSmem<G>& S, const int lane_g, Ac& a, bool alive, int nac, const EnvParams& P, float horizon,
                                          const uint16_t* s_pairs, int& nconf_env, int& nlos_env, const bool emit, const int e,
                                          const bool lane_moved, const double lat_ref, const double lon_ref) {
     const int lane = threadIdx.x & 31;
     const int wbase = lane - lane_g;                  // first lane of this group in the warp
-#ifdef BSG_SUBSTEP_CLOCKS
-    const bool clk_on = e == 0 && lane_g == 0 && horizon == 4.0f * P.simdt;
-#endif
-    BSG_CLK(0);
     // cos / sin of lat/2 from the cached cos(lat): half-angle identities (absolute error ~1e-7); sign of lat from its high word
     const float ch = sqrt_approx(fmaf(0.5f, a.coslat, 0.5f));
     const float sh = __int_as_float((__float_as_int(sqrt_approx(fmaxf(fmaf(-0.5f, a.coslat, 0.5f), 0.0f))) & 0x7fffffff) |
@@ -585,7 +565,7 @@ __device__ __forceinline__ void group_cd(GroupSmem<G>& S, const int lane_g, Ac& 
     bool moved;
     if (TOL) moved = ring && (fabsf(a.gse - hot[HU * 2 * G + (lane_g - 1)]) + fabsf(a.gsn - hot[HV * 2 * G + (lane_g - 1)]) > kCdVelTol);
     else moved = ring && lane_moved;
-    const bool eval_b = !BSG_CD_REUSE || P.cd_enabled == 2 || nb < 0 || __any_sync(gm, moved);
+    const bool eval_b = P.cd_enabled == 2 || nb < 0 || __any_sync(gm, moved);
     u64 KAP = 0, RR = 0, D0 = 0, DW = 0, LH = 0;
     if (eval_b) {
         if (ring) {
@@ -599,7 +579,7 @@ __device__ __forceinline__ void group_cd(GroupSmem<G>& S, const int lane_g, Ac& 
         if (lane_g == 0) S.cnt = 0;
         // allowances for keeping the list over `horizon` seconds (see the header comment)
         float kap = 0.0f, d0 = 0.0f, dw = 0.0f;
-        if (BSG_CD_REUSE && P.cd_enabled != 2 && horizon > 0.0f) {
+        if (P.cd_enabled != 2 && horizon > 0.0f) {
             const bool in = lane_g < nac;
             const float spd = in ? sqrtf(fmaf(a.gse, a.gse, a.gsn * a.gsn)) : 0.0f;
             // tan |lat| from the cached cos(lat) (capped near the poles like tan(89 deg))
@@ -616,7 +596,6 @@ __device__ __forceinline__ void group_cd(GroupSmem<G>& S, const int lane_g, Ac& 
         LH = pk2(lh, lh);
     }
     __syncwarp(gm);
-    BSG_CLK(1);
     if (eval_b) {
         // ---- (B) hot phase ---------------------------------------------------------------------------
         unsigned cand = 0u;
@@ -625,7 +604,7 @@ __device__ __forceinline__ void group_cd(GroupSmem<G>& S, const int lane_g, Ac& 
             const u64 nU = pk2(-a.gse, -a.gse), nV = pk2(-a.gsn, -a.gsn);
             const u64 EPS = pk2(kCdAbsEps, kCdAbsEps);
             const float* q = hot + r + 1;
-#pragma unroll kHotUnroll
+#pragma unroll 1
             for (int kk = 0; kk < kmax; kk += 2, q += 2) {        // offsets k = kk + 1 and kk + 2
                 const u64 nX = pk2(q[HX * 2 * G], q[HX * 2 * G + 1]);
                 const u64 Y = pk2(q[HY * 2 * G], q[HY * 2 * G + 1]);
@@ -682,7 +661,6 @@ __device__ __forceinline__ void group_cd(GroupSmem<G>& S, const int lane_g, Ac& 
         }
         if (lane_g == 0) S.nb = nb;
     }
-    BSG_CLK(2);
     // ---- (A) pairs with slot 0, every substep ----------------------------------------------------------------
     int ncand;
     {
@@ -701,17 +679,12 @@ __device__ __forceinline__ void group_cd(GroupSmem<G>& S, const int lane_g, Ac& 
         ncand = nb + __popc(bm);
         __syncwarp(gm);
     }
-    BSG_CLK(3);
     // ---- exact phase -------------------------------------------------------------------------------
     for (int p = lane_g; p < ncand; p += G) {
         const unsigned en = queue[p];
         exact_pair((int)(en >> 8), (int)(en & 0xffu));
     }
     found = ncand > 0;
-#ifdef BSG_SUBSTEP_CLOCKS
-    if (clk_on) g_clk[8] = ncand;
-#endif
-    BSG_CLK(4);
     }
     // one REDUX.OR over the group merges every lane's findings; each aircraft then reads its own bit
     if (found) {                                      // (group-uniform)
@@ -723,7 +696,6 @@ __device__ __forceinline__ void group_cd(GroupSmem<G>& S, const int lane_g, Ac& 
     nconf_env = counts & 0xffff;
     nlos_env = counts >> 16;
     __syncwarp(group_mask<G>());
-    BSG_CLK(5);
 }
 
 }  // namespace bsg

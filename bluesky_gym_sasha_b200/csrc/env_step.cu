@@ -2,9 +2,6 @@
 // termination, and the env-step megakernel that strings them around the substep loop of
 // env_kernels.cuh.  Every function cites the reference lines it restates; the float64 CPU
 // restatement these are parity-tested against is oracle/envs.py.
-#ifdef BSG_SUBSTEP_CLOCKS
-#include <cstdio>
-#endif
 #include "env_kernels.cuh"
 
 namespace bsg {
@@ -80,8 +77,8 @@ __device__ inline void descent_info(const EnvS& s, float* info) {           // d
 // HorizontalCREnv (horizontal_cr_env.py) -- slot 0 = ownship, slots 1..n = creconfs intruders
 // =====================================================================================================
 // The generator of an env that finishes runs at the END of a launch, on one warp, when the rest of the batch is done:
-// its dependent chain of float64 special functions IS the tail of the launch (25 us of a 45 us launch before this form;
-// scripts/phase_timing.py).  So: the ISA / CAS conversions at the configured altitude come from the host (init_tas0),
+// its dependent chain of float64 special functions IS the tail of the launch (25 us of a 45 us launch before this form,
+// measured with per-warp phase stamps).  So: the ISA / CAS conversions at the configured altitude come from the host (init_tas0),
 // upstream's vtas2cas -> cre -> vcas2tas round trip of an intruder's speed is taken as the identity it is (the intruder
 // flies the reference ground speed to 2e-16: |cas - 150| ~ 1e-14 << half an ulp of the float32 state), headings come from
 // the track angle instead of atan2 of its own sine / cosine, sines and cosines are evaluated in pairs (sincos), and the
@@ -894,26 +891,6 @@ __device__ __forceinline__ void do_info(const EnvS& s, const EnvParams& P, const
 // =====================================================================================================
 // K6: the env-step megakernel (also serves reset and the kinematics-only parity entry point)
 // =====================================================================================================
-// Phase stamps of a profiling build (-DBSG_PHASE_TIMING, scripts/phase_timing.py): %globaltimer at the phase boundaries of
-// every env's lane 0, parked in the unused tail of the final_obs buffer.  Not compiled into the product library.
-#ifndef BSG_FAST_STEADY
-#define BSG_FAST_STEADY 1
-#endif
-#ifndef BSG_PIN_SLOT
-#define BSG_PIN_SLOT 0
-#endif
-#ifndef BSG_PIN_GROUP
-#define BSG_PIN_GROUP 1
-#endif
-#ifndef BSG_TARGET_CACHE
-#define BSG_TARGET_CACHE 1
-#endif
-#ifdef BSG_PHASE_TIMING
-#define BSG_STAMP(k) do { asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(stamps[k]) :: "memory"); } while (0)
-#else
-#define BSG_STAMP(k) do { } while (0)
-#endif
-
 template <int ENV, int G, bool WIND>
 __global__ void __launch_bounds__(kEnvThreads, kEnvBlocksPerSm) env_kernel(const EnvParams P) {
     __shared__ GroupSmem<(G > 1) ? G : 2> s_grp[(G > 1) ? kEnvThreads / G : 1];
@@ -933,26 +910,16 @@ __global__ void __launch_bounds__(kEnvThreads, kEnvBlocksPerSm) env_kernel(const
         P.final_count[2] = P.fc_slot;
     }
     const int e = gt / G;
-    int slot_ = gt % G;
-#if BSG_PIN_SLOT
-    asm volatile("" : "+r"(slot_));
-#endif
-    const int slot = slot_;
+    const int slot = gt % G;
     if (e >= P.E) return;                       // group-uniform (G divides the block size)
     double* scratch = (ENV == BSG_ENV_SECTOR_CR) ? &s_scratch[(threadIdx.x / 32) * kSectorScratch]
                     : (ENV == BSG_ENV_STATIC_OBSTACLE) ? &s_scratch[(threadIdx.x / G) * kStaticScratch] : s_scratch;
     // (group index made opaque: otherwise the compiler, short of registers, rebuilds the group's shared-memory address from
     // the thread index -- S2R, shift, multiply-add -- at most of the dozen places per substep that use it)
     int grp = (G > 1) ? tid / G : 0;
-#if BSG_PIN_GROUP
     asm volatile("" : "+r"(grp));
-#endif
     auto& S = s_grp[grp];
 
-#ifdef BSG_PHASE_TIMING
-    unsigned long long stamps[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-#endif
-    BSG_STAMP(0);
     // Every load of the step is issued here, before anything waits on one of them: with the state cold in DRAM (the usual
     // case: 14 MB per batch touched once per env step) the aircraft record, the env counters and the actions arrive in ONE
     // memory round trip instead of three dependent ones, and the records read after the substep loop are on their way to L2.
@@ -989,7 +956,7 @@ __global__ void __launch_bounds__(kEnvThreads, kEnvBlocksPerSm) env_kernel(const
         // what they are a function of -- alt, vs, selspd, selalt -- stays put: the record carries allow_tas with a valid bit
         // that the end of a launch sets when its last targets belong to the stored (alt, vs), and that an action which
         // moves selspd / selalt clears.  Same inputs, same function: the cached value is the recomputed one bit for bit.
-        bool tgt_cached = (BSG_TARGET_CACHE && P.mode == kModeStep && (a.flags & kFlTgt) != 0) || !alive;   // (empty slots: nothing to compute)
+        bool tgt_cached = (P.mode == kModeStep && (a.flags & kFlTgt) != 0) || !alive;   // (empty slots: nothing to compute)
         if (P.mode == kModeStep) {
             const float o_selspd = a.selspd, o_selalt = a.selalt;
             if (ENV == BSG_ENV_DESCENT || ENV == BSG_ENV_VERTICAL_CR) descent_action<G>(a, P, act, slot);
@@ -1012,18 +979,16 @@ __global__ void __launch_bounds__(kEnvThreads, kEnvBlocksPerSm) env_kernel(const
             if (slot == 0) S.nb = -1;
             __syncwarp(group_mask<G>());
         }
-        BSG_STAMP(1);
         // (the envs whose action reads traf.cas convert tas -> cas after the loop and need the atmosphere for it)
         constexpr bool kNeedAtmos = ENV == BSG_ENV_SECTOR_CR || ENV == BSG_ENV_MERGE || ENV == BSG_ENV_STATIC_OBSTACLE;
         Targets T;
         compute_targets<kNeedAtmos>(a, P, T, tgt_cached);
-        BSG_STAMP(2);
         // `fixed`: the last full kinematics update left (tas, hdg, vs, alt, ax, ground-speed components) exactly as they
         // were.  They are a pure function of themselves, the targets T (recomputed only when alt / vs move) and the
         // commands (which change only between env steps, or through LNAV in MergeEnv, or with the wind): the next update
         // would reproduce them bit for bit, so while EVERY aircraft of the env is fixed -- intruders always, the ownship
         // once it has finished its turn -- a substep only advances the positions, with the very expressions of
-        // ac_kinematics (BSG_FAST_STEADY=0 switches the shortcut off: identical outputs, scripts/ab_identical.py).
+        // ac_kinematics.
         bool fixed = false;
         bool moved = false;                                 // the ground-speed vector changed in the last update (K3's (B) list)
 #pragma unroll 1
@@ -1044,10 +1009,7 @@ __global__ void __launch_bounds__(kEnvThreads, kEnvBlocksPerSm) env_kernel(const
                                                           nlos, emit, e, moved, lat_ref, lon_ref);
                 if (emit && slot == 0) P.ei32[(long long)e * BSG_I32_COUNT + BSG_I32_NPAIRS] = S.np;
             }
-#ifdef BSG_SUBSTEP_CLOCKS
-            if (e == 0 && slot == 0 && k == P.n_sub - 5) g_clk[6] = clock64();
-#endif
-            if (BSG_FAST_STEADY && !WIND && ENV != BSG_ENV_MERGE && group_all<G>(fixed || !alive)) {
+            if (!WIND && ENV != BSG_ENV_MERGE && group_all<G>(fixed || !alive)) {
                 moved = false;
                 if (alive) {                                // update_pos alone (same expressions as ac_kinematics)
                     a.lat += (double)(kRad2Deg * (P.simdt * a.gsn * (1.0f / kRearth)));
@@ -1060,23 +1022,11 @@ __global__ void __launch_bounds__(kEnvThreads, kEnvBlocksPerSm) env_kernel(const
                 moved = a.gsn != o_gsn || a.gse != o_gse;
                 fixed = !moved && a.tas == o_tas && a.hdg == o_hdg && a.vs == o_vs && a.alt == o_alt && a.ax == o_ax;
             }
-#ifdef BSG_SUBSTEP_CLOCKS
-            if (e == 0 && slot == 0 && k == P.n_sub - 5) {
-                g_clk[7] = clock64();
-                printf("substep clocks [cycles]: record+sync %lld | (B) %lld | (A) filter %lld | exact (%lld cand) %lld | merge+readback %lld | to kin %lld | kinematics %lld | whole %lld\n",
-                       g_clk[1] - g_clk[0], g_clk[2] - g_clk[1], g_clk[3] - g_clk[2], g_clk[8], g_clk[4] - g_clk[3], g_clk[5] - g_clk[4],
-                       g_clk[6] - g_clk[5], g_clk[7] - g_clk[6], g_clk[7] - g_clk[0]);
-            }
-#endif
             if (ENV == BSG_ENV_STATIC_OBSTACLE && P.mode == kModeStep) {   // per-substep reward / termination
                 if (k == 0) env_load_post(s, P, e);
                 if (static_substep_check<G>(a, s, P, e, slot)) break;
             }
-#ifdef BSG_PHASE_TIMING
-            if (k == 0) BSG_STAMP(3);
-#endif
         }
-        BSG_STAMP(4);
         // update_airspeed's cas = vtas2cas(tas, alt) uses the altitude from before update_pos: T.at of the last substep
         // (only the envs whose action reads traf.cas need it: Sector, Merge, StaticObstacle)
         if ((kNeedAtmos || P.mode == kModeTraf) && alive && P.n_sub > 0) {
@@ -1084,7 +1034,7 @@ __global__ void __launch_bounds__(kEnvThreads, kEnvBlocksPerSm) env_kernel(const
         }
         // targets cache for the next launch: valid when the last targets belong to the state that is stored
         a.tgt = T.allow_tas;
-        a.flags = (BSG_TARGET_CACHE && alive && T.k_alt == a.alt && T.k_vs == a.vs) ? (a.flags | kFlTgt) : (a.flags & ~kFlTgt);
+        a.flags = (alive && T.k_alt == a.alt && T.k_vs == a.vs) ? (a.flags | kFlTgt) : (a.flags & ~kFlTgt);
         s.nconf = nconf; s.nlos = nlos;
         if (P.mode == kModeTraf) {
             ac_store(a, P, gt);
@@ -1106,9 +1056,6 @@ __global__ void __launch_bounds__(kEnvThreads, kEnvBlocksPerSm) env_kernel(const
             obs[P.obs_dim - 2] = (wn * ch + we * sh) * (1.0f / 50.0f);
             obs[P.obs_dim - 1] = (-wn * sh + we * ch) * (1.0f / 50.0f);
         }
-#ifdef BSG_PHASE_TIMING
-        if (pass == 0) BSG_STAMP(5);
-#endif
         if (pass == 1) break;                            // SAME_STEP: the step's reward / flags / info stay
         if (fresh) {
             if (slot == 0) { P.reward[e] = 0.0f; P.term[e] = 0; P.trunc[e] = 0; do_info<ENV>(s, P, e); }
@@ -1134,19 +1081,8 @@ __global__ void __launch_bounds__(kEnvThreads, kEnvBlocksPerSm) env_kernel(const
         }
         resetting = true;
     }
-    BSG_STAMP(6);
     ac_store(a, P, gt);
     if (slot == 0) env_store(s, P, e);
-#ifdef BSG_PHASE_TIMING
-    BSG_STAMP(7);
-    if (slot == 0 && P.final_obs && P.mode == kModeStep) {
-        unsigned long long* out = reinterpret_cast<unsigned long long*>(P.final_obs + (long long)P.E * P.obs_dim) - 8LL * P.E;
-        unsigned smid;
-        asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-        stamps[7] = (stamps[7] & ~0xffULL) | (smid & 0xffu);      // SM id in the low byte of the last stamp (ns resolution lost: 256 ns)
-        for (int k = 0; k < 8; ++k) out[8LL * e + k] = stamps[k];
-    }
-#endif
 }
 
 }  // namespace bsg

@@ -241,10 +241,8 @@ __global__ void traf_conf_scatter_kernel(const TrafParams P) {
     }
 }
 
-#ifndef BSG_TRAF_MINBLOCKS
-#define BSG_TRAF_MINBLOCKS 6          // (<= 85 registers, no spills: 61 vs 68 us at 2^20 aircraft, 14.3 vs 16.4 us at 100k)
-#endif
-__global__ void __launch_bounds__(128, BSG_TRAF_MINBLOCKS) traf_substep_kernel(const TrafParams P) {
+// 6 CTAs per SM (<= 85 registers, no spills): 61 vs 68 us at 2^20 aircraft, 14.3 vs 16.4 us at 100k
+__global__ void __launch_bounds__(128, 6) traf_substep_kernel(const TrafParams P) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= P.n) return;
     if (!(P.flags[i] & BSG_TF_ALIVE)) return;

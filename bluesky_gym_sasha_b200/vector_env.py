@@ -9,7 +9,7 @@ libbsg_b200.so through the C ABI of include/bsg.h.  There is no CPU path.
 Two ways to drive it:
   * ``reset()`` / ``step(actions)``      -- numpy in / numpy float64 out (gymnasium, SB3, RLlib);
     each step copies actions host->device and obs / reward / flags / info device->host
-    (``bsg_step_host``).
+    (``bsg_step_host_block``).
   * ``reset_torch()`` / ``step_torch(a)`` -- CUDA float32 tensors in / out, no host sync.
 """
 import ctypes as C

@@ -20,8 +20,8 @@ t0 = time.perf_counter()
 for _ in range(500):
     v.step(a)
 torch.cuda.synchronize()
-print("chunks=%s threads=%s mode=%s copy=True : %.1f us" % (os.environ.get("BSG_D2H_CHUNKS", "4"), os.environ.get("BSG_HOST_THREADS", "4"),
-                                                        v.autoreset_mode, (time.perf_counter() - t0) / 500 * 1e6))
+print("threads=%s mode=%s copy=True : %.1f us" % (os.environ.get("BSG_HOST_THREADS", "4"), v.autoreset_mode,
+                                                 (time.perf_counter() - t0) / 500 * 1e6))
 v.copy = False
 t0 = time.perf_counter()
 for _ in range(500):

@@ -596,7 +596,7 @@ def test_soak_many_episodes_stay_finite(cuda, env_id, kw):
                                             ("SectorCREnv-v0", {}, 5), ("MergeEnv-v0", {}, 10)])
 def test_in_group_cd_kept_candidates_are_a_superset(cuda, env_id, kw, nsub):
     """K3 keeps the candidate list of the pairs among the un-steered aircraft across the substeps of an env step while
-    they hold their velocity (env_kernels.cuh, BSG_CD_REUSE).  cd_enabled=2 redoes the filter in every substep with no
+    they hold their velocity (env_kernels.cuh, group_cd).  cd_enabled=2 redoes the filter in every substep with no
     allowance; both must give bit-identical results -- after every substep count (bsg_traf_update with n = 1 .. n_sub
     from saved states, so a list kept for 1 .. n_sub - 1 substeps is compared), and along whole rollouts."""
     import torch
