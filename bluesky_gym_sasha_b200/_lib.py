@@ -60,6 +60,9 @@ CD_ATTR = ("qdr", "dist", "dcpa", "tcpa", "tinconf")          # BSG_CD_ATTR_* co
 # single-airspace traffic (bsg_traf_*): BSG_TF_* flag bits, BSG_TRAF_* sizes
 (TF_ALIVE, TF_LNAV, TF_VNAV, TF_VNAVSPD, TF_LASTWP, TF_ASAS, TF_RESOOFF, TF_PH_GD, TF_PH_AP, TF_ACTIVATE) = (1 << b for b in range(10))
 TF_IWP_SHIFT, TF_NWP_SHIFT, TRAF_PARTNERS, TRAF_CTR_COUNT = 16, 24, 8, 4
+# conflict / LoS event tracking (bsg_traf_events_*): BSG_EV_CTR_* slots of the counter array
+(EV_CTR_NCONF_TOTAL, EV_CTR_NLOS_TOTAL, EV_CTR_NCONF_ACTIVE, EV_CTR_NLOS_ACTIVE, EV_CTR_LOG_OVERFLOW, EV_CTR_TRUNCATED) = range(6)
+EV_CTR_COUNT = 8
 PRIM_LINE, PRIM_RING, PRIM_RECT, PRIM_EDGE, PRIM_EDGE_END, PRIM_FLOATS = 1, 2, 3, 4, 5, 8      # bsg_render records
 
 
@@ -72,6 +75,12 @@ class TrafConfig(C.Structure):
 class TrafTensors(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in ("pos", "kin", "cmd", "aux", "actwp", "vnav1", "vnav2", "asas", "flags", "partners",
                                           "rt_pos", "rt_con", "rt_dir", "counters")]
+
+
+class TrafEvents(C.Structure):
+    _fields_ = [("d_cur", C.c_void_p), ("d_prev", C.c_void_p), ("set_bytes", C.c_int64), ("d_conf_log", C.c_void_p),
+                ("d_los_log", C.c_void_p), ("d_los_sev", C.c_void_p), ("conf_log_cap", C.c_int64), ("los_log_cap", C.c_int64),
+                ("d_counters", C.c_void_p)]
 
 
 class Layout(C.Structure):
@@ -92,7 +101,8 @@ class TensorTable(C.Structure):
 SYMBOLS = ("bsg_abi_version", "bsg_abi_struct_size", "bsg_last_error", "bsg_device_count", "bsg_query_layout", "bsg_create",
            "bsg_destroy", "bsg_bind_state", "bsg_reset", "bsg_step", "bsg_step_host", "bsg_step_host_block", "bsg_step_host_copy", "bsg_step_host_begin", "bsg_step_host_wait", "bsg_host_copy", "bsg_host_widen", "bsg_set_obs_noise", "bsg_get_noise_calls", "bsg_set_noise_calls", "bsg_load_state", "bsg_set_seed", "bsg_set_wind", "bsg_traf_update",
            "bsg_cd_padded", "bsg_cd_pack", "bsg_cd_order_workspace", "bsg_cd_pack_ordered", "bsg_cd_detect", "bsg_cd_cull_workspace", "bsg_cd_detect_culled", "bsg_cd_detect_peers", "bsg_probe_fp32",
-           "bsg_traf_pack", "bsg_traf_activate", "bsg_traf_workspace", "bsg_traf_substep", "bsg_render")
+           "bsg_traf_pack", "bsg_traf_activate", "bsg_traf_workspace", "bsg_traf_substep", "bsg_traf_events_workspace",
+           "bsg_traf_events_update", "bsg_render")
 
 _lib = None
 
@@ -152,6 +162,9 @@ def load():
     lib.bsg_traf_substep.argtypes = [C.POINTER(TrafConfig), C.POINTER(TrafTensors), vp, i32, vp, vp, vp, vp, i64, vp, i64, vp]
     lib.bsg_traf_workspace.argtypes = [i64, i64]
     lib.bsg_traf_workspace.restype = i64
+    lib.bsg_traf_events_workspace.argtypes = [i64, i64]
+    lib.bsg_traf_events_workspace.restype = i64
+    lib.bsg_traf_events_update.argtypes = [C.POINTER(TrafEvents), vp, C.POINTER(CdLists), i64, vp]
     lib.bsg_cd_padded.argtypes = [i64]
     lib.bsg_cd_padded.restype = i64
     lib.bsg_cd_pack.argtypes = [vp, vp, vp, vp, vp, vp, i64, f64, f64, vp, vp]
@@ -167,10 +180,10 @@ def load():
     lib.bsg_abi_struct_size.argtypes = [C.c_int]
     lib.bsg_abi_struct_size.restype = C.c_int
     for name in ("bsg_query_layout", "bsg_create", "bsg_bind_state", "bsg_reset", "bsg_step", "bsg_step_host", "bsg_step_host_block", "bsg_step_host_copy",
-                 "bsg_traf_update", "bsg_traf_pack", "bsg_traf_activate", "bsg_traf_substep", "bsg_cd_pack", "bsg_cd_pack_ordered",
+                 "bsg_traf_update", "bsg_traf_pack", "bsg_traf_activate", "bsg_traf_substep", "bsg_traf_events_update", "bsg_cd_pack", "bsg_cd_pack_ordered",
                  "bsg_cd_detect", "bsg_cd_detect_culled", "bsg_cd_detect_peers", "bsg_probe_fp32"):
         getattr(lib, name).restype = C.c_int
-    for which, st in enumerate((Config, Layout, TensorTable, Wind, Perf, AcState, CdLists, TrafConfig, TrafTensors)):
+    for which, st in enumerate((Config, Layout, TensorTable, Wind, Perf, AcState, CdLists, TrafConfig, TrafTensors, TrafEvents)):
         if lib.bsg_abi_struct_size(which) != C.sizeof(st):
             raise BsgError(f"{LIB_PATH}: sizeof({st.__name__}) is {lib.bsg_abi_struct_size(which)} in the library, "
                            f"{C.sizeof(st)} in bluesky_gym_sasha_b200/_lib.py (include/bsg.h changed: rebuild / update the binding)")

@@ -9,7 +9,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.environ.get("BSG_LIB_OUT") or os.path.join(HERE, "libbsg_b200.so")      # BSG_LIB_OUT: A/B builds
-SOURCES = ["api.cu", "env_step.cu", "cd_tiled.cu", "host_pool.cu", "obs_noise.cu", "traf_airspace.cu", "render.cu", "cd_order.cu"]
+SOURCES = ["api.cu", "env_step.cu", "cd_tiled.cu", "host_pool.cu", "obs_noise.cu", "traf_airspace.cu", "traf_events.cu", "render.cu", "cd_order.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared", "--expt-relaxed-constexpr"]
 

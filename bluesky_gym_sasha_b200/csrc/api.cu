@@ -65,6 +65,7 @@ extern "C" int bsg_abi_struct_size(int which) {
         case 6: return (int)sizeof(bsg_cd_lists);
         case 7: return (int)sizeof(bsg_traf_config);
         case 8: return (int)sizeof(bsg_traf_tensors);
+        case 9: return (int)sizeof(bsg_traf_events);
     }
     return -1;
 }

@@ -5,6 +5,8 @@ Interface mirrored: the handful of ``bs.traf`` / ``bs.stack`` calls a BlueSky sc
 select commands, ``RESO MVP`` / ``RESO OFF`` (``reso=``; the reference's own line is ``reso off``, merge_env.py:157),
 ``RESOOFF acid``, ``bs.sim.step()`` (``step``) -- with the state arrays ``lat, lon, alt, tas, hdg, vs, ...`` as properties.
 Per substep: ``bsg_traf_pack`` -> ``bsg_cd_detect[_culled]`` with pair lists (K2) -> ``bsg_traf_substep`` (include/bsg.h).  Restated for checking in oracle/traffic_ext.py.  No CPU fallback.
+With ``events=True`` each detection also feeds ``bsg_traf_events_update``: the conflict / LoS event counts and logs of
+upstream's ConflictDetection.update (``conflict_counts``, ``conflict_log``; restated in oracle/conflict_log.py).
 """
 import ctypes as C
 
@@ -95,11 +97,19 @@ class AirspaceTraffic:
 
     def __init__(self, n_max, device=0, simdt=1.0, rpz=5.0 * NM, hpz=1000.0 * FT, dtlookahead=300.0, reso=None, reso_mode=0,
                  resofach=1.01, resofacv=1.01, perf=None, max_wpts=8, lat0=52.0, lon0=4.0, cull=True, symmetric=True,
-                 pair_capacity=None, fms_dt=10.5, group=None):
+                 pair_capacity=None, fms_dt=10.5, group=None, events=False, event_capacity=None):
         """``group``: a ``torch.distributed`` process group (``True`` = the default group) over which ONE airspace is sharded,
         one rank per GPU (SURVEY 8e): every rank owns the kinematics of up to ``n_max`` aircraft (its block); per substep the
         ranks all-gather their CD records (32 B per aircraft over NVLink), each detects the conflicts of its own rows against
-        the whole airspace and advances its own aircraft.  Results equal the unsharded airspace's."""
+        the whole airspace and advances its own aircraft.  Results equal the unsharded airspace's.
+
+        ``events=True``: every detection also updates the conflict and LoS event record of upstream's
+        ConflictDetection.update (confpairs_all / lospairs_all) on the device (bsg_traf_events_update), read with
+        ``conflict_counts()`` and ``conflict_log()``.  ``event_capacity``: rows of each event log (default 8 x n_max); the
+        totals stay exact when a log is full.  Not with ``group``: on a row-sharded rank the two orders of a pair sit on
+        different GPUs, so counting unordered pairs would need an exchange of the pair lists."""
+        if events and group is not None and group is not False:
+            raise ValueError("events=True is not available for an airspace sharded over a process group")
         if not torch.cuda.is_available():
             raise _lib.BsgError("AirspaceTraffic needs a CUDA device: there is no CPU fallback")
         if reso not in (None, "OFF", "MVP"):
@@ -134,6 +144,20 @@ class AirspaceTraffic:
         self.work = torch.zeros(int(self.lib.bsg_traf_workspace(n, cap)), dtype=torch.uint8, device=dev)      # (zeroed once)
         self.last = None                    # device outputs of the last substep's detection
         self.gpu_launches = 0
+        self.events = bool(events)
+        if self.events:
+            ecap = int(event_capacity) if event_capacity is not None else 8 * self.n_max
+            if ecap < 0:
+                raise ValueError("event_capacity must be >= 0")
+            nb = int(self.lib.bsg_traf_events_workspace(cap, cap))
+            self.ev_sets = [torch.zeros(nb, dtype=torch.uint8, device=dev) for _ in range(2)]    # (zeroed once)
+            rows = max(ecap, 1)
+            self.ev = dict(conf_log=z(rows, 4, dt=torch.int32), los_log=z(rows, 4, dt=torch.int32), los_sev=z(rows, 2),
+                           counters=z(_lib.EV_CTR_COUNT, dt=torch.int64))
+            self.ev_struct = _lib.TrafEvents(set_bytes=nb, d_conf_log=_ptr(self.ev["conf_log"]), d_los_log=_ptr(self.ev["los_log"]),
+                                             d_los_sev=_ptr(self.ev["los_sev"]), conf_log_cap=ecap, los_log_cap=ecap,
+                                             d_counters=_ptr(self.ev["counters"]))
+            self.event_capacity = ecap
         # one airspace over several GPUs: block k of the records belongs to rank k, `per` records each (whole tiles)
         self.group, self.world, self.rank, self.row0 = None, 1, 0, 0
         if group is not None and group is not False:
@@ -269,6 +293,8 @@ class AirspaceTraffic:
                         out = cd.detect_packed(rec, n, want_pairs=True, cull=self.cull, symmetric=self.symmetric)
                     self.last = out
                     self.gpu_launches += 1
+                    if self.events:
+                        self._track_events(out, st)
                     if self.reso:
                         pairs, attr, npairs = out["pairs"], out["attr"], out["npairs"]
                         self.gpu_launches += 3
@@ -277,6 +303,16 @@ class AirspaceTraffic:
                                                      cd.pair_capacity if pairs is not None else 0,
                                                      _ptr(self.work), self.work.numel(), st))
                 self.gpu_launches += 1
+
+    def _track_events(self, out, st):
+        """bsg_traf_events_update on this detection's lists, then the sets swap roles."""
+        ev, cd = self.ev_struct, self.cd
+        ev.d_cur, ev.d_prev = _ptr(self.ev_sets[0]), _ptr(self.ev_sets[1])
+        lists = _lib.CdLists(d_conf_pairs=_ptr(out["pairs"]), d_conf_attr=_ptr(out["attr"]), conf_cap=cd.pair_capacity,
+                             d_los_pairs=_ptr(out["lospairs"]), los_cap=cd.los_capacity, d_npairs=_ptr(out["npairs"]))
+        _lib.check(self.lib.bsg_traf_events_update(C.byref(ev), _ptr(self.rec), C.byref(lists), self.nstep, st))
+        self.ev_sets.reverse()
+        self.gpu_launches += 2
 
     # ------------------------------------------------------------------ state (device tensors, views)
     def _col(self, name, c):
@@ -318,4 +354,29 @@ class AirspaceTraffic:
                    truncated=n_conf > self.cd.pair_capacity or n_los > self.cd.los_capacity)
         for c, name in enumerate(_lib.CD_ATTR):
             res[name] = attr[o, c].astype(np.float64)
+        return res
+
+    def conflict_counts(self):
+        """Event totals since creation (``events=True``): ``nconf_total`` = len(confpairs_all), ``nlos_total`` =
+        len(lospairs_all), the events open after the last detection (``nconf_active``, ``nlos_active``), ``log_overflow``
+        (events not logged: log full) and ``truncated`` (detections whose pair lists were incomplete, npairs > pair_capacity:
+        from the first one on, the events are unreliable).  Copies only the counter array."""
+        if not self.events:
+            raise _lib.BsgError("AirspaceTraffic was created without events=True")
+        c = self.ev["counters"].cpu().numpy()
+        keys = ("nconf_total", "nlos_total", "nconf_active", "nlos_active", "log_overflow", "truncated")
+        return {k: int(c[i]) for i, k in enumerate(keys)}
+
+    def conflict_log(self):
+        """Host copy of the event logs (``events=True``), sorted by (start, a, b): ``confpairs_all`` [m, 2] (a < b),
+        ``conf_start``, ``conf_end`` (the ``nstep`` of the first detection with / without the pair; end -1 = still open),
+        ``lospairs_all`` [k, 2], ``los_start``, ``los_end``, ``los_dmin`` / ``los_dalt_min`` [m] (least horizontal distance /
+        |dalt| over the event's detections), and the counts of ``conflict_counts()``.  The time of step s is (s - 1) * simdt."""
+        res = self.conflict_counts()
+        mc, ml = min(res["nconf_total"], self.event_capacity), min(res["nlos_total"], self.event_capacity)
+        conf, los = self.ev["conf_log"][:mc].cpu().numpy(), self.ev["los_log"][:ml].cpu().numpy()
+        sev = self.ev["los_sev"][:ml].cpu().numpy().astype(np.float64)
+        o, ol = np.lexsort((conf[:, 1], conf[:, 0], conf[:, 2])), np.lexsort((los[:, 1], los[:, 0], los[:, 2]))
+        res.update(confpairs_all=conf[o, :2], conf_start=conf[o, 2], conf_end=conf[o, 3], lospairs_all=los[ol, :2],
+                   los_start=los[ol, 2], los_end=los[ol, 3], los_dmin=sev[ol, 0], los_dalt_min=sev[ol, 1])
         return res

@@ -143,7 +143,7 @@ typedef struct bsg_handle bsg_handle;
 
 int bsg_abi_version(void);
 /* sizeof of the library's view of an interface structure (which: 0 bsg_config, 1 bsg_layout, 2 bsg_tensor_table,
- * 3 bsg_wind, 4 bsg_perf, 5 bsg_ac_state, 6 bsg_cd_lists, 7 bsg_traf_config, 8 bsg_traf_tensors; anything else -1): a binding in another language checks its own declarations against it */
+ * 3 bsg_wind, 4 bsg_perf, 5 bsg_ac_state, 6 bsg_cd_lists, 7 bsg_traf_config, 8 bsg_traf_tensors, 9 bsg_traf_events; anything else -1): a binding in another language checks its own declarations against it */
 int bsg_abi_struct_size(int which);
 const char *bsg_last_error(void);
 int bsg_device_count(void);
@@ -409,6 +409,39 @@ int64_t bsg_traf_workspace(int64_t n, int64_t conf_cap);
 int bsg_traf_substep(const bsg_traf_config *cfg, const bsg_traf_tensors *t, const float *d_rec, int32_t fms_ready,
                      const int32_t *d_conf_pairs, const float *d_conf_attr, const unsigned long long *d_npairs,
                      const unsigned long long *d_nconf_all, int64_t conf_cap, void *d_work, int64_t work_bytes, void *stream);
+
+/* ---- conflict and loss-of-separation events of an airspace -------------------------------------------------------
+ * Replaces the bookkeeping of upstream's ConflictDetection.update (bluesky/traffic/asas/detection.py): confpairs_all /
+ * lospairs_all, i.e. the number of conflicts and LoS of an experiment, plus per event its start / end and, for LoS, its
+ * severity.  Call bsg_traf_events_update once per detection, after bsg_cd_detect[_culled] on the same stream, with that
+ * detection's lists.  An event is an UNORDERED pair (a < b) that is in the detection's conflict (LoS) list in either order;
+ * it starts at the first detection that lists it after one that did not and ends (end = nstep) at the first later
+ * detection that does not.  LoS events keep the minimum horizontal distance and |dalt| [m] over their detections, from
+ * d_rec with cd_pair.cuh's algebra.  Totals count every event even when its log is full (rows beyond the capacity are
+ * dropped and counted in BSG_EV_CTR_LOG_OVERFLOW); a detection with npairs > cap (lists incomplete) increments
+ * BSG_EV_CTR_TRUNCATED, after which the log is unreliable.  Lists of one airspace on one GPU with global indices (not the
+ * row-sharded form: there the two orders of a pair sit on different GPUs).  Asynchronous: no host synchronisation.
+ * Stateless: everything lives in the caller-owned DEVICE memory below. */
+enum { BSG_EV_CTR_NCONF_TOTAL = 0, BSG_EV_CTR_NLOS_TOTAL = 1 /* events so far (= log rows claimed) */,
+       BSG_EV_CTR_NCONF_ACTIVE = 2, BSG_EV_CTR_NLOS_ACTIVE = 3 /* events open after the last detection */,
+       BSG_EV_CTR_LOG_OVERFLOW = 4 /* events not logged (log full) */, BSG_EV_CTR_TRUNCATED = 5 /* detections with npairs > cap */,
+       BSG_EV_CTR_COUNT = 8 };
+typedef struct bsg_traf_events {
+    void *d_cur;                /* set of this detection: set_bytes, 16-byte aligned                                      */
+    void *d_prev;               /* set of the previous detection.  Both ZERO before the first call; the call leaves d_prev
+                                 * zero again, so the caller swaps d_cur and d_prev after every call                       */
+    int64_t set_bytes;          /* >= bsg_traf_events_workspace(conf_cap, los_cap) of the lists (the same caps every call) */
+    int32_t *d_conf_log;        /* [conf_log_cap][4] a, b, start nstep, end nstep (-1 while open); row = event number      */
+    int32_t *d_los_log;         /* [los_log_cap][4] the same for LoS events                                                */
+    float *d_los_sev;           /* [los_log_cap][2] dmin, dalt_min [m]                                                     */
+    int64_t conf_log_cap, los_log_cap;
+    unsigned long long *d_counters; /* [BSG_EV_CTR_COUNT], zero before the first call                                   */
+} bsg_traf_events;
+/* Bytes of ONE set (a hash table of >= 2 x (conf_cap + los_cap) 16-byte slots and the dense list of its occupied slots). */
+int64_t bsg_traf_events_workspace(int64_t conf_cap, int64_t los_cap);
+/* d_rec: the records the detection ran on (needed with a LoS list); nstep: the simulator step of the detection, stored as
+ * start / end.  Launches a memset and two kernels. */
+int bsg_traf_events_update(const bsg_traf_events *ev, const float *d_rec, const bsg_cd_lists *lists, int64_t nstep, void *stream);
 
 /* ---- rgb_array frames (SURVEY 8f-4) --------------------------------------------------------------------------------
  * Paints a list of draw calls into an RGB frame on the device: d_prims [n_prims][BSG_PRIM_FLOATS] float32 records
