@@ -13,6 +13,9 @@ BSG_OK, BSG_EINVAL, BSG_ECUDA, BSG_ESTATE, BSG_ENOMEM = 0, -1, -2, -3, -4
 ENV_DESCENT, ENV_HORIZONTAL_CR, ENV_SECTOR_CR, ENV_MERGE, ENV_PLAN_WAYPOINT, ENV_VERTICAL_CR, ENV_STATIC_OBSTACLE = 0, 1, 2, 3, 4, 5, 6
 AUTORESET_DISABLED, AUTORESET_NEXT_STEP, AUTORESET_SAME_STEP = 0, 1, 2
 CD_LON_WRAP, CD_SYMMETRIC, CD_CULL, CD_ALLTILES = 1, 2, 4, 8
+# CD record storage [tile][field][CD_TILE] (BSG_CD_TILE, BSG_CD_REC_*)
+CD_TILE = 256
+CD_REC_X, CD_REC_Y, CD_REC_CH, CD_REC_SH, CD_REC_U, CD_REC_V, CD_REC_ALT, CD_REC_VS, CD_REC_FIELDS = range(9)
 
 # indices into the per-env records (include/bsg.h)
 F64_WPT_LAT, F64_WPT_LON, F64_TARGET_ALT, F64_POLY_AREA, F64_WPTS, F64_COUNT = 0, 1, 2, 3, 4, 16

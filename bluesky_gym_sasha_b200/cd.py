@@ -21,6 +21,56 @@ def _ptr(t):
     return C.c_void_p(t.data_ptr()) if t is not None else C.c_void_p(0)
 
 
+def cd_records(n, device, inert=False):
+    """CD records for ``n`` aircraft (include/bsg.h: BSG_CD_TILE, BSG_CD_REC_*): a float32 tensor
+    [tiles, CD_REC_FIELDS, CD_TILE] holding bsg_cd_padded(n) records, at least one tile.  ``inert=True``: every record
+    starts as the inert padding record bsg_cd_pack writes (alt 3e9: never a conflict candidate)."""
+    tiles = max(int(_lib.load().bsg_cd_padded(n)) // _lib.CD_TILE, 1)
+    rec = (torch.zeros if inert else torch.empty)((tiles, _lib.CD_REC_FIELDS, _lib.CD_TILE), dtype=torch.float32, device=device)
+    if inert:
+        rec[:, _lib.CD_REC_CH, :] = 1.0
+        rec[:, _lib.CD_REC_ALT, :] = 3.0e9
+    return rec
+
+
+def all_gather_records(rec_local, n_local, group=None, out=None):
+    """The first ``n_local`` records of every rank's ``rec_local`` (whole tiles), all-gathered in rank order: the records
+    of ``n_local * world`` aircraft.  ``out``: the buffer of an earlier call, reused when it is large enough."""
+    import torch.distributed as dist
+    assert n_local % _lib.CD_TILE == 0, "shard size must be a multiple of the 256-aircraft tile"
+    tiles = n_local // _lib.CD_TILE
+    world = dist.get_world_size(group)
+    if out is None or out.shape[0] < tiles * world:
+        out = cd_records(n_local * world, rec_local.device)
+    dist.all_gather_into_tensor(out[:tiles * world], rec_local[:tiles].contiguous(), group=group)
+    return out
+
+
+def host_lists(out, lists, per_aircraft, perm=None):
+    """Host form of a detection's pair lists (``detect_packed`` with ``want_pairs``; ``lists``: its ``StateBasedCD.lists``),
+    as upstream's detect() returns them: ``confpairs``, ``lospairs`` (up to the lists' capacity, row-major order), the
+    host arrays of ``per_aircraft``, ``n_conf``, ``n_los``, ``truncated`` (more pairs found than the lists hold), ``qdr,
+    dist, dcpa, tcpa, tinconf`` per conflict.  ``perm``: record k holds aircraft ``perm[k]`` (``pack_ordered``).
+    Synchronises the device."""
+    torch.cuda.synchronize(out["npairs"].device)
+    n_conf, n_los = (int(v) for v in out["npairs"].cpu())
+    k, kl = min(n_conf, lists.conf_cap), min(n_los, lists.los_cap)
+    pairs, lospairs, attr = out["pairs"][:k], out["lospairs"][:kl], out["attr"][:k]
+    if perm is not None:
+        pairs = perm[pairs.long()].to(torch.int32)
+        lospairs = perm[lospairs.long()].to(torch.int32)
+    # upstream's order: row-major np.where (own index, then intruder index).  Keys are unique, so one sort of the
+    # combined 64-bit key on the device orders a list
+    o = torch.argsort(pairs[:, 0].long() * (1 << 32) + pairs[:, 1].long())
+    ol = torch.argsort(lospairs[:, 0].long() * (1 << 32) + lospairs[:, 1].long())
+    attr = attr[o].cpu().numpy().astype(np.float64)
+    res = dict(confpairs=pairs[o].cpu().numpy(), lospairs=lospairs[ol].cpu().numpy(), **per_aircraft,
+               n_conf=n_conf, n_los=n_los, truncated=n_conf > lists.conf_cap or n_los > lists.los_cap)
+    for c, name in enumerate(_lib.CD_ATTR):           # qdr, dist, dcpa, tcpa, tinconf of each conflict (detect()'s tail)
+        res[name] = attr[:, c]
+    return res
+
+
 class StateBasedCD:
     def __init__(self, device=0, rpz=5.0 * NM, hpz=1000.0 * FT, dtlookahead=300.0, pair_capacity=1 << 22,
                  los_capacity=None):
@@ -33,6 +83,7 @@ class StateBasedCD:
         self.los_capacity = int(pair_capacity if los_capacity is None else los_capacity)
         self.gpu_launches = 0
         self._buf = {}
+        self.lists = None                   # bsg_cd_lists of the last detection (_lists)
 
     def _stream(self):
         return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
@@ -51,11 +102,10 @@ class StateBasedCD:
 
     # ---------------------------------------------------------------- packing
     def pack(self, lat, lon, trk, gs, alt, vs, lat0, lon0, out=None):
-        """float64 SoA -> tile-blocked float32 CD records [n_pad/256, 8, 256] (padding = inert aircraft)."""
+        """float64 SoA -> CD records (``cd_records``; padding = inert aircraft)."""
         arrs = [self._as_dev(a) for a in (lat, lon, trk, gs, alt, vs)]
         n = arrs[0].numel()
-        n_pad = int(self.lib.bsg_cd_padded(n))
-        rec = out if out is not None else torch.empty((max(n_pad // 256, 1), 8, 256), dtype=torch.float32, device=self.device)
+        rec = out if out is not None else cd_records(n, self.device)
         with torch.cuda.device(self.device):
             _lib.check(self.lib.bsg_cd_pack(*[_ptr(a) for a in arrs], n, float(lat0), float(lon0), _ptr(rec),
                                             self._stream()))
@@ -68,8 +118,7 @@ class StateBasedCD:
         aircraft ``perm[k]`` (int32 device tensor)."""
         arrs = [self._as_dev(a) for a in (lat, lon, trk, gs, alt, vs)]
         n = arrs[0].numel()
-        n_pad = int(self.lib.bsg_cd_padded(n))
-        rec = out if out is not None else torch.empty((max(n_pad // 256, 1), 8, 256), dtype=torch.float32, device=self.device)
+        rec = out if out is not None else cd_records(n, self.device)
         perm = torch.empty((n,), dtype=torch.int32, device=self.device)
         nbytes = int(self.lib.bsg_cd_order_workspace(n))
         work = self._get("order_work", (nbytes,), torch.uint8)
@@ -81,13 +130,15 @@ class StateBasedCD:
 
     # ---------------------------------------------------------------- detection on packed records
     def _lists(self, want_pairs, want_attr=True):
-        """Device pair lists of one detection (include/bsg.h::bsg_cd_lists) and the ctypes view handed to the library."""
+        """Device pair lists of one detection (include/bsg.h::bsg_cd_lists) and the ctypes view handed to the library, which
+        also stays in ``self.lists``."""
         npairs = self._get("npairs", (2,), torch.int64)
         pairs = self._get("pairs", (max(self.pair_capacity, 1), 2), torch.int32) if want_pairs else None
         attr = self._get("attr", (max(self.pair_capacity, 1), len(_lib.CD_ATTR)), torch.float32) if want_pairs and want_attr else None
         los = self._get("lospairs", (max(self.los_capacity, 1), 2), torch.int32) if want_pairs else None
         lists = _lib.CdLists(d_conf_pairs=_ptr(pairs), d_conf_attr=_ptr(attr), conf_cap=self.pair_capacity if want_pairs else 0,
                              d_los_pairs=_ptr(los), los_cap=self.los_capacity if want_pairs else 0, d_npairs=_ptr(npairs))
+        self.lists = lists
         return lists, dict(pairs=pairs, attr=attr, lospairs=los, npairs=npairs)
 
     def detect_packed(self, rec, n_all, row0=0, n_rows=None, lon_wrap=False, want_pairs=True, cull=False, symmetric=False,
@@ -95,6 +146,7 @@ class StateBasedCD:
         """Rows [row0, row0+n_rows) x all n_all columns.  Asynchronous; returns device tensors: per-row ``nconf_row``,
         ``nlos_row``, ``tcpamax``, ``inconf``; ``npairs`` = (conflicts, LoS pairs) found; with ``want_pairs`` the lists
         ``pairs`` [cap, 2] (+ ``attr`` [cap, 5] = qdr, dist, dcpa, tcpa, tinconf per conflict) and ``lospairs`` [cap, 2].
+        ``self.lists`` holds the ``_lib.CdLists`` view of those lists that the detection wrote.
         ``cull=True``: bsg_cd_detect_culled (identical outputs; pays off on spatially sorted records).
         ``symmetric=True`` (full N x N only): each unordered tile pair is evaluated once and both ordered results are
         emitted (BSG_CD_SYMMETRIC; identical outputs, half the pair evaluations); combines with ``cull``."""
@@ -173,33 +225,18 @@ class StateBasedCD:
         else:
             rec, n = self.pack(lat_d, lon_d, trk, gs, alt, vs, lat0, lon0)
         out = self.detect_packed(rec, n, lon_wrap=span >= 90.0, cull=cull, symmetric=symmetric and span < 90.0)
-        torch.cuda.synchronize(self.device)
-        n_conf, n_los = (int(v) for v in out["npairs"].cpu())
-        k, kl = min(n_conf, self.pair_capacity), min(n_los, self.los_capacity)
-        pairs, lospairs, attr = out["pairs"][:k], out["lospairs"][:kl], out["attr"][:k]
         inconf, tcpamax = out["inconf"], out["tcpamax"]
         nconf_row, nlos_row = out["nconf_row"], out["nlos_row"]
         if perm is not None:                              # back to the caller's aircraft order
-            pairs = perm[pairs.long()].to(torch.int32)
-            lospairs = perm[lospairs.long()].to(torch.int32)
             def unperm(x):
                 y = torch.empty_like(x)
                 y[perm] = x
                 return y
             inconf, tcpamax, nconf_row, nlos_row = (unperm(x) for x in (inconf, tcpamax, nconf_row, nlos_row))
-        # upstream's order: row-major np.where (own index, then intruder index).  Keys are unique, so one sort of the
-        # combined 64-bit key on the device (plumbing of this convenience wrapper, after the detection) orders a list
-        o = torch.argsort(pairs[:, 0].long() * (1 << 32) + pairs[:, 1].long())
-        ol = torch.argsort(lospairs[:, 0].long() * (1 << 32) + lospairs[:, 1].long())
-        attr = attr[o].cpu().numpy().astype(np.float64)
-        res = dict(confpairs=pairs[o].cpu().numpy(), lospairs=lospairs[ol].cpu().numpy(), inconf=inconf.cpu().numpy().astype(bool),
-                   tcpamax=tcpamax.cpu().numpy().astype(np.float64),
-                   nconf_row=nconf_row.cpu().numpy().astype(np.int64),
-                   nlos_row=nlos_row.cpu().numpy().astype(np.int64),
-                   n_conf=n_conf, n_los=n_los, truncated=n_conf > self.pair_capacity or n_los > self.los_capacity)
-        for c, name in enumerate(_lib.CD_ATTR):           # qdr, dist, dcpa, tcpa, tinconf of each conflict (detect()'s tail)
-            res[name] = attr[:, c]
-        return res
+        return host_lists(out, self.lists, dict(inconf=inconf.cpu().numpy().astype(bool),
+                                                tcpamax=tcpamax.cpu().numpy().astype(np.float64),
+                                                nconf_row=nconf_row.cpu().numpy().astype(np.int64),
+                                                nlos_row=nlos_row.cpu().numpy().astype(np.int64)), perm)
 
     # ---------------------------------------------------------------- multi-GPU: rows sharded over ranks
     def detect_sharded(self, rec_local, n_local, group=None, lon_wrap=False, want_pairs=False, cull=False):
@@ -210,9 +247,7 @@ class StateBasedCD:
         import torch.distributed as dist
         world = dist.get_world_size(group)
         rank = dist.get_rank(group)
-        assert n_local % 256 == 0, "shard size must be a multiple of the 256-aircraft tile"
-        allrec = self._get("allrec", (n_local // 256 * world, 8, 256), torch.float32)
-        dist.all_gather_into_tensor(allrec, rec_local[:n_local // 256].contiguous(), group=group)
+        allrec = self._buf["allrec"] = all_gather_records(rec_local, n_local, group, self._buf.get("allrec"))
         return self.detect_packed(allrec, n_local * world, row0=rank * n_local, n_rows=n_local,
                                   lon_wrap=lon_wrap, want_pairs=want_pairs, cull=cull)
 
@@ -225,9 +260,7 @@ class StateBasedCD:
         ``npairs`` holds the global totals.  Pair lists (``want_pairs``) stay partitioned by tile-pair owner."""
         import torch.distributed as dist
         world, rank = dist.get_world_size(group), dist.get_rank(group)
-        assert n_local % 256 == 0, "shard size must be a multiple of the 256-aircraft tile"
-        allrec = self._get("allrec", (n_local // 256 * world, 8, 256), torch.float32)
-        dist.all_gather_into_tensor(allrec, rec_local[:n_local // 256].contiguous(), group=group)
+        allrec = self._buf["allrec"] = all_gather_records(rec_local, n_local, group, self._buf.get("allrec"))
         out = self.detect_packed(allrec, n_local * world, want_pairs=want_pairs, cull=cull, symmetric=True, deal=(world, rank))
         counts = self._get("sym_counts", (2, n_local * world), torch.int32)
         counts[0].copy_(out["nconf_row"])
@@ -250,16 +283,17 @@ class StateBasedCD:
         import torch.distributed._symmetric_memory as symm
         group = group if group is not None else dist.group.WORLD
         world, rank = dist.get_world_size(group), dist.get_rank(group)
-        assert n_local % 256 == 0 and world <= 8, "shard size must be a multiple of 256; one node (<= 8 GPUs)"
+        assert n_local % _lib.CD_TILE == 0 and world <= 8, "shard size must be a multiple of 256; one node (<= 8 GPUs)"
+        local = rec_local[:n_local // _lib.CD_TILE]
         st = self._buf.get("symm")
         if st is None or st[0] != n_local:
-            buf = symm.empty((n_local // 256, 8, 256), dtype=torch.float32, device=self.device)
+            buf = symm.empty(local.shape, dtype=torch.float32, device=self.device)
             hdl = symm.rendezvous(buf, group)
             ptrs = (C.c_void_p * world)(*[int(p) for p in hdl.buffer_ptrs])
             st = (n_local, buf, hdl, ptrs)
             self._buf["symm"] = st
         _, buf, hdl, ptrs = st
-        buf.copy_(rec_local[:n_local // 256])
+        buf.copy_(local)
         hdl.barrier(channel=0)                  # every rank's block is in place (device-side, on the current stream)
         m = n_local
         nconf = self._get("nconf", (m,), torch.int32)

@@ -67,7 +67,7 @@ __device__ __forceinline__ void order_grid(const OrderWork* w, long long n, doub
     const double la1 = dunkey(w->box[1]), o1 = dunkey(w->box[3]);
     const double h = fmax(la1 - la0, 1e-9);
     const double wd = fmax((o1 - o0) * cos(0.5 * (la0 + la1) * 0.017453292519943295), 1e-9);
-    const double tiles = fmax(1.0, ceil((double)n / 256.0));
+    const double tiles = fmax(1.0, ceil((double)n / (double)BSG_CD_TILE));
     double strips = fmax(1.0, rint(sqrt(tiles * h / wd)));
     strips = fmin(strips, 512.0);
     double bins = fmax(1.0, ceil(tiles / strips * (double)kBinsPerTile));

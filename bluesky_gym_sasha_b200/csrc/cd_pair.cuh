@@ -3,7 +3,7 @@
 // (see oracle/statebased.py for the float64 restatement this is checked against; the reference never
 // enables ASAS -- merge_env.py:157 only issues `reso off` -- BASELINE.json's north_star adds it).
 //
-// CD record (32 B, two float4):  A = (x, y, ch, sh)   B = (u, v, alt, vs)
+// CD record (32 B, two float4; stored tile-blocked, cd_record.cuh):  A = (x, y, ch, sh)   B = (u, v, alt, vs)
 //   x = Re*rad(lon - lon0), y = Re*rad(lat - lat0)   [m of arc from the airspace origin]
 //   ch, sh = cos, sin of lat/2                       (cos of the pair's mean latitude = chi*chj - shi*shj)
 //   u = gs sin(trk), v = gs cos(trk)                 [m/s east, north]

@@ -10,9 +10,8 @@
 // column *pairs* (j, j+1): 26 packed FMA-pipe ops per two pairs + 13 scalar ALU/MUFU ops per pair
 // (~28 issue slots and 26 FMA-pipe clk per ordered pair, vs 56 issue slots for the scalar formulation).
 //
-// Layout: records are tile-blocked SoA -- rec[tile][field 0..7][256] floats (field = x, y, ch, sh, u, v,
-// alt, vs; see cd_pair.cuh) -- so a column tile is one contiguous 8 KB block that the TMA engine copies
-// into shared memory (cp.async.bulk + mbarrier complete_tx, two stages; SASS UBLKCP) and a broadcast
+// Layout: records are tile-blocked SoA (cd_record.cuh), so a column tile is one contiguous 8 KB block that the TMA
+// engine copies into shared memory (cp.async.bulk + mbarrier complete_tx, two stages; SASS UBLKCP) and a broadcast
 // LDS.128 yields two ready-made packed operands (j..j+1, j+2..j+3) of one field.
 // Decomposition: work item = (256 own rows) x (8 column tiles); a persistent grid of (SMs x resident
 // CTAs) strides over the items, so the tail is < 1 item.  The hot loop only decides "conflict candidate";
@@ -25,10 +24,10 @@
 #include "bsg_internal.h"
 #include "bsg_math.cuh"
 #include "cd_pair.cuh"
+#include "cd_record.cuh"
 
 namespace bsg {
 
-constexpr int kTJ = 256;                 // columns per tile
 constexpr int kNT = 128;                 // threads per CTA
 constexpr int kR = 2;                    // rows per thread
 constexpr int kRowsPerCta = kNT * kR;    // 256 = one tile of rows
@@ -36,9 +35,7 @@ constexpr int kTilesPerItem = 8;          // upper bound; the launch picks fewer
 // culled form: work item = one row block x up to kTilesPerChunk listed column tiles.  Measured at N = 100k (2.8 % of
 // the tile pairs kept): 1 -> 0.506 ms, 2 -> 0.539, 4 -> 0.574, 8 -> 0.626: balance beats the per-item set-up cost.
 constexpr int kTilesPerChunk = 1;
-constexpr int kTileFloats = 8 * kTJ;
 constexpr uint32_t kTileBytes = kTileFloats * 4;
-enum { FX = 0, FY = 1, FCH = 2, FSH = 3, FU = 4, FV = 5, FALT = 6, FVS = 7 };
 
 typedef unsigned long long u64;
 
@@ -99,8 +96,9 @@ struct CdArgs {
     int deal_n, deal_k;           // BSG_CD_DEAL: only the row blocks with (row tile % deal_n) == deal_k (0, 0: all)
 };
 
+// record idx as cd_pair.cuh's two halves A = (x, y, ch, sh), B = (u, v, alt, vs)
 __device__ __forceinline__ void load_record(const float* __restrict__ rec, int idx, float4& A, float4& B) {
-    const float* t = rec + (size_t)(idx / kTJ) * kTileFloats + (idx % kTJ);
+    const float* t = cd_rec(rec, idx);
     A = make_float4(t[FX * kTJ], t[FY * kTJ], t[FCH * kTJ], t[FSH * kTJ]);
     B = make_float4(t[FU * kTJ], t[FV * kTJ], t[FALT * kTJ], t[FVS * kTJ]);
 }
@@ -212,7 +210,7 @@ __device__ __forceinline__ void cd_process_item(const CdArgs& a, float (*s_tile)
     const int tid = threadIdx.x;
     auto tile_of = [&](int tt) { return LIST ? (int)list[tt] : t_begin + tt; };
     const int own_tile = a.row0 / kRowsPerCta + rb;          // (SYM: rows are tile-aligned)
-    // own rows -> packed registers.  Rows past the shard end are made inert (alt -3e9: can never be a
+    // own rows -> packed registers.  Rows past the shard end are made inert (alt -kInertAlt: can never be a
     // candidate), so the hot loop needs no validity test.
     RowPack rp[kR];
     int ri[kR];
@@ -225,7 +223,7 @@ __device__ __forceinline__ void cd_process_item(const CdArgs& a, float (*s_tile)
         ri[k] = r;
         float4 A, B;
         load_record(a.rec_rows, (r < row_end ? r : row_end - 1) - a.rows_base, A, B);
-        if (r >= row_end) B.z = -3.0e9f;                // inert row (padding columns sit at +3e9)
+        if (r >= row_end) B.z = -kInertAlt;             // inert row (padding columns sit at +kInertAlt)
         rp[k].nX = pk2(-A.x, -A.x); rp[k].nY = pk2(-A.y, -A.y);
         rp[k].CH = pk2(A.z, A.z);   rp[k].nSH = pk2(-A.w, -A.w);
         rp[k].nU = pk2(-B.x, -B.x); rp[k].nV = pk2(-B.y, -B.y);
@@ -499,7 +497,7 @@ __global__ void cd_finalize_kernel(const uint32_t* __restrict__ nconf_row, uint8
     if (i < n) inconf[i] = nconf_row[i] > 0;
 }
 
-// float64 SoA -> tile-blocked float32 records (see cd_pair.cuh); padding entries are inert aircraft.
+// float64 SoA -> CD records (cd_record.cuh); padding entries are inert aircraft.
 __global__ void cd_pack_kernel(const double* __restrict__ lat, const double* __restrict__ lon,
                                const double* __restrict__ trk, const double* __restrict__ gs,
                                const double* __restrict__ alt, const double* __restrict__ vs,
@@ -507,26 +505,17 @@ __global__ void cd_pack_kernel(const double* __restrict__ lat, const double* __r
                                long long n_pad, double lat0, double lon0, float* __restrict__ rec) {
     const long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x;      // record index
     if (k >= n_pad) return;
-    float f[8];
+    float f[BSG_CD_REC_FIELDS];
     if (k < n) {
         const long long i = perm ? (long long)perm[k] : k;                     // the aircraft it holds (bsg_cd_pack_ordered)
-        double la = lat[i];
-        double dl = fmod((lon[i] - lon0) + 180.0, 360.0);
-        if (dl < 0.0) dl += 360.0;
-        dl -= 180.0;
-        double s, c, st, ct;
-        sincos(la * (0.5 * kDeg2RadD), &s, &c);
+        cd_rec_position(f, lat[i], lon[i], lat0, lon0);
+        double st, ct;
         sincos(trk[i] * kDeg2RadD, &st, &ct);
-        f[FX] = (float)(kRearthD * kDeg2RadD * dl); f[FY] = (float)(kRearthD * kDeg2RadD * (la - lat0));
-        f[FCH] = (float)c; f[FSH] = (float)s;
         f[FU] = (float)(gs[i] * st); f[FV] = (float)(gs[i] * ct); f[FALT] = (float)alt[i]; f[FVS] = (float)vs[i];
     } else {
-        f[FX] = 0.0f; f[FY] = 0.0f; f[FCH] = 1.0f; f[FSH] = 0.0f;
-        f[FU] = 0.0f; f[FV] = 0.0f; f[FALT] = 3.0e9f; f[FVS] = 0.0f;   // |dalt| ~ 3e9: never a candidate
+        cd_rec_inert(f);
     }
-    float* t = rec + (size_t)(k / kTJ) * kTileFloats + (k % kTJ);
-#pragma unroll
-    for (int q = 0; q < 8; ++q) t[q * kTJ] = f[q];
+    cd_rec_store(rec, k, f);
 }
 
 }  // namespace bsg

@@ -17,13 +17,11 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "cd_record.cuh"
 #include "env_kernels.cuh"
 
 namespace bsg {
 
-constexpr int kTJ2 = 256;                       // aircraft per CD record tile (cd_tiled.cu: kTJ)
-constexpr int kTileFloats2 = 8 * kTJ2;
-enum { RX = 0, RY = 1, RCH = 2, RSH = 3, RU = 4, RV = 5, RALT = 6, RVS = 7 };
 constexpr float kSteepness = 3000.0f * kFt / (10.0f * kNm);        // Autopilot.steepness
 
 struct TrafParams {
@@ -51,10 +49,6 @@ struct TrafAc {
     float ap_alt;                 // Autopilot.alt of this substep (ComputeVNAV may dial it in)
     uint32_t f;                   // BSG_TF_*
 };
-
-__device__ __forceinline__ float rec_at(const float* rec, long long j, int field) {
-    return rec[(j / kTJ2) * kTileFloats2 + field * kTJ2 + (j % kTJ2)];
-}
 
 // Autopilot.ComputeVNAV (swtod = swtoc = True, no RTA): once per leg.  dist2wp [m] to the active waypoint.
 __device__ __forceinline__ void compute_vnav(Ac& a, TrafAc& x, const float toalt, const float xtoalt, const float dist2wp) {
@@ -137,24 +131,17 @@ __device__ __forceinline__ void traf_store(const Ac& a, const TrafAc& x, const T
 __global__ void traf_pack_kernel(const TrafParams P, float* __restrict__ rec, const long long n_pad) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_pad) return;
-    float f[8] = {0.0f, 0.0f, 1.0f, 0.0f, 0.0f, 0.0f, 3.0e9f, 0.0f};       // padding / dead slots: inert (|dalt| ~ 3e9)
+    float f[BSG_CD_REC_FIELDS];
+    cd_rec_inert(f);                                                        // padding / dead slots
     if (i < P.n && (P.flags[i] & BSG_TF_ALIVE)) {
         const double2 p = P.pos[i];
         const float4 k = P.kin[i];
-        double dl = fmod((p.y - P.lon0) + 180.0, 360.0);
-        if (dl < 0.0) dl += 360.0;
-        dl -= 180.0;
-        double s, c;
-        sincos(p.x * (0.5 * kDeg2RadD), &s, &c);
+        cd_rec_position(f, p.x, p.y, P.lat0, P.lon0);
         float sh, ch;
         sincosf(k.z * kDeg2Rad, &sh, &ch);
-        f[RX] = (float)(kRearthD * kDeg2RadD * dl); f[RY] = (float)(kRearthD * kDeg2RadD * (p.x - P.lat0));
-        f[RCH] = (float)c; f[RSH] = (float)s;
-        f[RU] = k.y * sh; f[RV] = k.y * ch; f[RALT] = k.x; f[RVS] = k.w;
+        f[FU] = k.y * sh; f[FV] = k.y * ch; f[FALT] = k.x; f[FVS] = k.w;
     }
-    float* t = rec + (size_t)(i / kTJ2) * kTileFloats2 + (i % kTJ2);
-#pragma unroll
-    for (int q = 0; q < 8; ++q) t[q * kTJ2] = f[q];
+    cd_rec_store(rec, i, f);
 }
 
 __global__ void traf_activate_kernel(const TrafParams P) {
@@ -316,7 +303,8 @@ __global__ void __launch_bounds__(128, 6) traf_substep_kernel(const TrafParams P
     // ---- ASAS: ConflictResolution.update = MVP.resolve (when the detection found any conflict) + resumenav -----------
     if (P.reso) {
         const long long ig = P.row0 + i;                   // this aircraft in the records of the whole airspace
-        const float own_u = rec_at(P.rec, ig, RU), own_v = rec_at(P.rec, ig, RV), own_alt = rec_at(P.rec, ig, RALT), own_vs = rec_at(P.rec, ig, RVS);
+        const float own_u = cd_rec_at(P.rec, ig, FU), own_v = cd_rec_at(P.rec, ig, FV);
+        const float own_alt = cd_rec_at(P.rec, ig, FALT), own_vs = cd_rec_at(P.rec, ig, FVS);
         const unsigned long long ntot = P.nconf_all[0];
         const int k0 = P.offs[i], k1 = k0 + P.len[i];
         // the aircraft's conflicts in ascending intruder order (its run of the index is unordered; runs are short)
@@ -336,8 +324,8 @@ __global__ void __launch_bounds__(128, 6) traf_substep_kernel(const TrafParams P
                 const float* q = P.attr + (long long)row * BSG_CD_ATTR_COUNT;
                 float e1, e2, e3, ts;
                 mvp_pair(P, q[BSG_CD_ATTR_QDR], q[BSG_CD_ATTR_DIST], q[BSG_CD_ATTR_TCPA], q[BSG_CD_ATTR_TINCONF],
-                         rec_at(P.rec, j, RALT) - own_alt, rec_at(P.rec, j, RU) - own_u, rec_at(P.rec, j, RV) - own_v,
-                         rec_at(P.rec, j, RVS) - own_vs, e1, e2, e3, ts);
+                         cd_rec_at(P.rec, j, FALT) - own_alt, cd_rec_at(P.rec, j, FU) - own_u, cd_rec_at(P.rec, j, FV) - own_v,
+                         cd_rec_at(P.rec, j, FVS) - own_vs, e1, e2, e3, ts);
                 tsolv_min = fminf(tsolv_min, ts);
                 d1 -= e1; d2 -= e2; d3 -= 0.5f * e3;      // cooperative: half the vertical part each
                 if (x.f & BSG_TF_RESOOFF) { d1 = 0.0f; d2 = 0.0f; d3 = 0.0f; }
@@ -389,16 +377,17 @@ __global__ void __launch_bounds__(128, 6) traf_substep_kernel(const TrafParams P
             }
         }
         bool any_pair = false, active = false;
-        const float own_x = rec_at(P.rec, ig, RX), own_y = rec_at(P.rec, ig, RY), own_ch = rec_at(P.rec, ig, RCH), own_sh = rec_at(P.rec, ig, RSH);
+        const float own_x = cd_rec_at(P.rec, ig, FX), own_y = cd_rec_at(P.rec, ig, FY);
+        const float own_ch = cd_rec_at(P.rec, ig, FCH), own_sh = cd_rec_at(P.rec, ig, FSH);
         const float own_trk = mod360(kRad2Deg * atan2f(own_u, own_v));
 #pragma unroll
         for (int s = 0; s < BSG_TRAF_PARTNERS; ++s) {
             const int j = part[s];
             if (j < 0) continue;
             any_pair = true;
-            const float cav = fmaf(-own_sh, rec_at(P.rec, j, RSH), own_ch * rec_at(P.rec, j, RCH));
-            const float dx = (rec_at(P.rec, j, RX) - own_x) * cav, dy = rec_at(P.rec, j, RY) - own_y;
-            const float ju = rec_at(P.rec, j, RU), jv = rec_at(P.rec, j, RV);
+            const float cav = fmaf(-own_sh, cd_rec_at(P.rec, j, FSH), own_ch * cd_rec_at(P.rec, j, FCH));
+            const float dx = (cd_rec_at(P.rec, j, FX) - own_x) * cav, dy = cd_rec_at(P.rec, j, FY) - own_y;
+            const float ju = cd_rec_at(P.rec, j, FU), jv = cd_rec_at(P.rec, j, FV);
             const bool past_cpa = fmaf(dx, ju - own_u, dy * (jv - own_v)) > 0.0f;
             const float hdist = sqrtf(fmaf(dx, dx, dy * dy));
             const bool hor_los = hdist < P.rpz;
@@ -499,7 +488,7 @@ extern "C" int bsg_traf_pack(const bsg_traf_config* cfg, const bsg_traf_tensors*
     int rc = traf_params(P, cfg, t, "bsg_traf_pack");
     if (rc != BSG_OK) return rc;
     if (!d_rec) return bsg_fail(BSG_EINVAL, "bsg_traf_pack: null d_rec");
-    const long long n_pad = ((P.n + kTJ2 - 1) / kTJ2) * kTJ2;
+    const long long n_pad = bsg_cd_padded(P.n);
     if (n_pad == 0) return BSG_OK;
     traf_pack_kernel<<<(unsigned)(n_pad / 256), 256, 0, (cudaStream_t)stream>>>(P, d_rec, n_pad);
     return bsg_cuda_check(cudaGetLastError(), "bsg_traf_pack launch");

@@ -21,10 +21,10 @@
 #include <stdint.h>
 
 #include "bsg_internal.h"
+#include "cd_record.cuh"
 
 namespace bsg {
 
-constexpr int kEvTile = 256;                    // aircraft per CD record tile (cd_tiled.cu: kTJ)
 constexpr int kEvThreads = 256;
 constexpr int64_t kEvMaxPairs = 1LL << 28;      // conf_cap + los_cap: slot indices of the tables stay below 2^30
 constexpr int64_t kEvHeader = 16;               // set header: uint32 number of occupied slots, padded to 16 bytes
@@ -74,20 +74,17 @@ __device__ __forceinline__ bool ev_find(const EvSlot* tab, const unsigned long l
     }
 }
 
-__device__ __forceinline__ float ev_rec(const float* rec, const int j, const int field) {
-    return rec[(size_t)(j / kEvTile) * (8 * kEvTile) + field * kEvTile + (j % kEvTile)];
-}
-
 // Horizontal distance and |dalt| of the pair (a, b) in this detection's CD records, cd_pair.cuh's algebra
 // (dx = dlon-difference * (ch_a ch_b - sh_a sh_b), dy = lat-difference).  Every step is an explicitly rounded IEEE
 // operation -- no contraction into FMAs -- so the value is exactly symmetric in a and b and a float32 restatement on the
 // host reproduces it bit for bit.
 __device__ __forceinline__ void ev_los_severity(const float* rec, const int a, const int b, float& d, float& dalt) {
-    const float cav = __fsub_rn(__fmul_rn(ev_rec(rec, a, 2), ev_rec(rec, b, 2)), __fmul_rn(ev_rec(rec, a, 3), ev_rec(rec, b, 3)));
-    const float dx = __fmul_rn(__fsub_rn(ev_rec(rec, b, 0), ev_rec(rec, a, 0)), cav);
-    const float dy = __fsub_rn(ev_rec(rec, b, 1), ev_rec(rec, a, 1));
+    const float cav = __fsub_rn(__fmul_rn(cd_rec_at(rec, a, FCH), cd_rec_at(rec, b, FCH)),
+                                __fmul_rn(cd_rec_at(rec, a, FSH), cd_rec_at(rec, b, FSH)));
+    const float dx = __fmul_rn(__fsub_rn(cd_rec_at(rec, b, FX), cd_rec_at(rec, a, FX)), cav);
+    const float dy = __fsub_rn(cd_rec_at(rec, b, FY), cd_rec_at(rec, a, FY));
     d = __fsqrt_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)));
-    dalt = fabsf(__fsub_rn(ev_rec(rec, b, 6), ev_rec(rec, a, 6)));
+    dalt = fabsf(__fsub_rn(cd_rec_at(rec, b, FALT), cd_rec_at(rec, a, FALT)));
 }
 
 __global__ void __launch_bounds__(kEvThreads) traf_ev_insert_kernel(const EvParams P) {

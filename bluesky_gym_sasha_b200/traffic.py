@@ -14,7 +14,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from .cd import StateBasedCD, _ptr
+from .cd import StateBasedCD, _ptr, all_gather_records, cd_records, host_lists
 
 NM, FT, FPM, KTS = 1852.0, 0.3048, 0.3048 / 60.0, 0.514444
 
@@ -139,8 +139,9 @@ class AirspaceTraffic:
                       rt_pos=z(n, W, 2, dt=torch.float64), rt_con=z(n, W, 4), rt_dir=z(n, W),
                       counters=z(_lib.TRAF_CTR_COUNT, dt=torch.int32))
         self.tt = _lib.TrafTensors(**{k: _ptr(v) for k, v in self.t.items()})
-        n_pad = int(self.lib.bsg_cd_padded(n))
-        self.rec = torch.empty((max(n_pad // 256, 1), 8, 256), dtype=torch.float32, device=dev)
+        sharded = group is not None and group is not False
+        # (sharded: records this rank never packs, beyond its aircraft count, stay inert)
+        self.rec = cd_records(n, dev, inert=sharded)
         self.work = torch.zeros(int(self.lib.bsg_traf_workspace(n, cap)), dtype=torch.uint8, device=dev)      # (zeroed once)
         self.last = None                    # device outputs of the last substep's detection
         self.gpu_launches = 0
@@ -160,17 +161,14 @@ class AirspaceTraffic:
             self.event_capacity = ecap
         # one airspace over several GPUs: block k of the records belongs to rank k, `per` records each (whole tiles)
         self.group, self.world, self.rank, self.row0 = None, 1, 0, 0
-        if group is not None and group is not False:
+        if sharded:
             import torch.distributed as dist
             self.group = None if group is True else group
             self.world, self.rank = dist.get_world_size(self.group), dist.get_rank(self.group)
-            self.per = max(n_pad, 256)
+            self.per = self.rec.shape[0] * _lib.CD_TILE
             self.row0 = self.rank * self.per
             self.cfg.row0 = self.row0
-            self.rec.zero_()                # records this rank never packs (beyond its aircraft count) stay inert
-            self.rec[:, 2, :] = 1.0
-            self.rec[:, 6, :] = 3.0e9
-            self.allrec = torch.empty((self.per // 256 * self.world, 8, 256), dtype=torch.float32, device=dev)
+            self.allrec = cd_records(self.per * self.world, dev)
             self.nconf_all = torch.zeros(2, dtype=torch.int64, device=dev)
 
     # ------------------------------------------------------------------ plumbing
@@ -282,8 +280,7 @@ class AirspaceTraffic:
                     _lib.check(self.lib.bsg_traf_pack(C.byref(self.cfg), C.byref(self.tt), _ptr(self.rec), st))
                     if self.world > 1:
                         import torch.distributed as dist
-                        dist.all_gather_into_tensor(self.allrec, self.rec[:self.per // 256], group=self.group)
-                        rec = self.allrec
+                        rec = self.allrec = all_gather_records(self.rec, self.per, self.group, self.allrec)
                         out = cd.detect_packed(rec, self.per * self.world, row0=self.row0, n_rows=n, want_pairs=True, cull=self.cull)
                         if self.reso:       # upstream resolves whenever ANY conflict exists in the airspace
                             self.nconf_all.copy_(out["npairs"])
@@ -294,7 +291,7 @@ class AirspaceTraffic:
                     self.last = out
                     self.gpu_launches += 1
                     if self.events:
-                        self._track_events(out, st)
+                        self._track_events(st)
                     if self.reso:
                         pairs, attr, npairs = out["pairs"], out["attr"], out["npairs"]
                         self.gpu_launches += 3
@@ -304,13 +301,11 @@ class AirspaceTraffic:
                                                      _ptr(self.work), self.work.numel(), st))
                 self.gpu_launches += 1
 
-    def _track_events(self, out, st):
+    def _track_events(self, st):
         """bsg_traf_events_update on this detection's lists, then the sets swap roles."""
-        ev, cd = self.ev_struct, self.cd
+        ev = self.ev_struct
         ev.d_cur, ev.d_prev = _ptr(self.ev_sets[0]), _ptr(self.ev_sets[1])
-        lists = _lib.CdLists(d_conf_pairs=_ptr(out["pairs"]), d_conf_attr=_ptr(out["attr"]), conf_cap=cd.pair_capacity,
-                             d_los_pairs=_ptr(out["lospairs"]), los_cap=cd.los_capacity, d_npairs=_ptr(out["npairs"]))
-        _lib.check(self.lib.bsg_traf_events_update(C.byref(ev), _ptr(self.rec), C.byref(lists), self.nstep, st))
+        _lib.check(self.lib.bsg_traf_events_update(C.byref(ev), _ptr(self.rec), C.byref(self.cd.lists), self.nstep, st))
         self.ev_sets.reverse()
         self.gpu_launches += 2
 
@@ -344,17 +339,8 @@ class AirspaceTraffic:
         out = self.last
         if out is None:
             raise _lib.BsgError("no detection has run yet")
-        torch.cuda.synchronize(self.device)
-        n_conf, n_los = (int(v) for v in out["npairs"].cpu())
-        k, kl = min(n_conf, self.cd.pair_capacity), min(n_los, self.cd.los_capacity)
-        pairs, los, attr = out["pairs"][:k].cpu().numpy(), out["lospairs"][:kl].cpu().numpy(), out["attr"][:k].cpu().numpy()
-        o, ol = np.lexsort((pairs[:, 1], pairs[:, 0])), np.lexsort((los[:, 1], los[:, 0]))
-        res = dict(confpairs=pairs[o], lospairs=los[ol], inconf=out["inconf"][:self.n].cpu().numpy().astype(bool),
-                   tcpamax=out["tcpamax"][:self.n].cpu().numpy().astype(np.float64), n_conf=n_conf, n_los=n_los,
-                   truncated=n_conf > self.cd.pair_capacity or n_los > self.cd.los_capacity)
-        for c, name in enumerate(_lib.CD_ATTR):
-            res[name] = attr[o, c].astype(np.float64)
-        return res
+        return host_lists(out, self.cd.lists, dict(inconf=out["inconf"][:self.n].cpu().numpy().astype(bool),
+                                                   tcpamax=out["tcpamax"][:self.n].cpu().numpy().astype(np.float64)))
 
     def conflict_counts(self):
         """Event totals since creation (``events=True``): ``nconf_total`` = len(confpairs_all), ``nlos_total`` =

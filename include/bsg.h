@@ -257,10 +257,16 @@ int bsg_traf_update(bsg_handle *h, int32_t n_sub, void *stream);
 
 /* ---- single-airspace state-based conflict detection (StateBased.detect; CD record = 32 B) -------- */
 
-/* Packs float64 SoA aircraft state (bs.traf.lat/lon/trk/gs/alt/vs) into 32-byte float CD records
- * (x, y metres from (lat0, lon0); cos/sin of half latitude; u, v; alt; vs), stored tile-blocked:
- * d_rec[tile][field 0..7][256] floats, tile = aircraft index / 256.  d_rec must hold bsg_cd_padded(n)
- * records (8 floats each); the padding of the last tile is filled with inert aircraft. */
+/* CD record storage, tile-blocked: d_rec[tile][BSG_CD_REC_FIELDS][BSG_CD_TILE] floats, tile = aircraft index /
+ * BSG_CD_TILE; field k of aircraft j is d_rec[(j / BSG_CD_TILE) * BSG_CD_TILE * BSG_CD_REC_FIELDS + k * BSG_CD_TILE +
+ * j % BSG_CD_TILE].  Fields: x, y [m of arc from (lat0, lon0)], ch, sh (cos, sin of half the latitude), u, v [m/s east,
+ * north], alt [m], vs [m/s].  Padding records are inert: ch = 1, alt = 3e9, every other field 0. */
+enum { BSG_CD_TILE = 256,
+       BSG_CD_REC_X = 0, BSG_CD_REC_Y = 1, BSG_CD_REC_CH = 2, BSG_CD_REC_SH = 3,
+       BSG_CD_REC_U = 4, BSG_CD_REC_V = 5, BSG_CD_REC_ALT = 6, BSG_CD_REC_VS = 7, BSG_CD_REC_FIELDS = 8 };
+
+/* Packs float64 SoA aircraft state (bs.traf.lat/lon/trk/gs/alt/vs) into 32-byte CD records (BSG_CD_REC_*).
+ * d_rec must hold bsg_cd_padded(n) records; the padding of the last tile is filled with inert aircraft. */
 int64_t bsg_cd_padded(int64_t n);
 int bsg_cd_pack(const double *d_lat, const double *d_lon, const double *d_trk, const double *d_gs,
                 const double *d_alt, const double *d_vs, int64_t n, double lat0, double lon0,

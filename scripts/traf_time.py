@@ -28,7 +28,7 @@ def staged_step(self):
         out = timed("detect", lambda: cd.detect_packed(self.rec, self.n, want_pairs=True, cull=self.cull, symmetric=self.symmetric))
         self.last = out
         if self.events:
-            timed("events", lambda: self._track_events(out, st))
+            timed("events", lambda: self._track_events(st))
         timed("substep", lambda: _lib.check(self.lib.bsg_traf_substep(C.byref(self.cfg), C.byref(self.tt), _ptr(self.rec), int(fms_ready),
               _ptr(out["pairs"]), _ptr(out["attr"]), _ptr(out["npairs"]), None, cd.pair_capacity, _ptr(self.work), self.work.numel(), st)))
 

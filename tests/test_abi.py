@@ -30,6 +30,16 @@ def test_header_symbols_exported(lib):
     assert lib.bsg_abi_struct_size(99) == -1
 
 
+def test_cd_record_constants_match_header():
+    """_lib's CD record constants (tile width, field indices) are the BSG_CD_TILE / BSG_CD_REC_* enum of include/bsg.h."""
+    from bluesky_gym_sasha_b200 import _lib
+    src = re.sub(r"/\*.*?\*/", "", open(os.path.join(ROOT, "include", "bsg.h")).read(), flags=re.S)
+    enum = dict(re.findall(r"\bBSG_(CD_TILE|CD_REC_[A-Z]+)\s*=\s*(\d+)", src))
+    assert sorted(enum) == sorted(["CD_TILE", "CD_REC_FIELDS"] + ["CD_REC_" + f for f in ("X", "Y", "CH", "SH", "U", "V", "ALT", "VS")])
+    for name, value in enum.items():
+        assert getattr(_lib, name) == int(value), name
+
+
 def test_layout_queries(lib):
     from bluesky_gym_sasha_b200 import _lib, spec
     want = {"DescentEnv-v0": (1, 4, 1, 30, 1.0), "HorizontalCREnv-v0": (8, 28, 1, 10, 5.0),

@@ -183,3 +183,18 @@ def test_sb3_lazy_infos_behave_like_a_list_of_dicts():
     assert len(lazy[1:4]) == 3
     lazy[2] = {"replaced": 1}                    # wrappers may overwrite entries
     assert lazy[2] == {"replaced": 1}
+
+
+def test_cd_records_allocator_shape_and_inert_padding(lib):
+    """cd.cd_records: bsg_cd_padded(n) records as [tiles, 8, 256] float32 (at least one tile); inert=True fills every
+    record with the padding record of bsg_cd_pack: x, y, sh, u, v, vs = 0, ch = 1, alt = 3e9."""
+    import torch
+    from bluesky_gym_sasha_b200.cd import cd_records
+    for n, tiles in ((0, 1), (1, 1), (256, 1), (257, 2), (100_000, 391)):
+        rec = cd_records(n, "cpu")
+        assert rec.shape == (tiles, 8, 256) and rec.dtype == torch.float32 and rec.device.type == "cpu"
+        inert = cd_records(n, "cpu", inert=True)
+        assert inert.shape == (tiles, 8, 256) and inert.dtype == torch.float32
+        want = np.zeros(8, np.float32)
+        want[2], want[6] = 1.0, 3.0e9
+        assert np.array_equal(inert.numpy(), np.broadcast_to(want[None, :, None], (tiles, 8, 256)))
