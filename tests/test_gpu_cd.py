@@ -14,12 +14,27 @@ pytestmark = pytest.mark.gpu
 RPZ, HPZ, DTL = 9260.0, 304.8, 300.0
 
 
-def _check_against_oracle(s, g, rows=None, stats=None, pos_quant=0.5):
+def _pos_quant(s, lat0=None, lon0=None):
+    """Twice the float32 step of the largest |x|, |y| of the packed CD records (the origin as StateBasedCD.detect picks it
+    by default): the resolution of the kernel's positions.  0.5 m within ~20 deg of the origin, 4 m half a world away."""
+    import torch
+    from bluesky_gym_sasha_b200 import _lib
+    from bluesky_gym_sasha_b200.cd import StateBasedCD
+    lat0 = float(np.mean(s[0])) if lat0 is None else lat0
+    lon0 = float(s[1][0]) if lon0 is None else lon0
+    rec, n = StateBasedCD().pack(*s, lat0, lon0)
+    xy = rec[:, [_lib.CD_REC_X, _lib.CD_REC_Y], :].permute(0, 2, 1).reshape(-1, 2)[:n]
+    return 2.0 * float(np.spacing(np.float32(xy.abs().max().item())))
+
+
+def _check_against_oracle(s, g, rows=None, stats=None, zone=(RPZ, HPZ, DTL), lat0=None, lon0=None):
     """Conflict AND LoS pair sets (as sets of ordered index pairs) identical to the float64 oracle outside the epsilon
-    band; per-row outputs for rows with no banded pair; qdr / dist / dcpa / tcpa / tinconf of every common conflict."""
+    band; per-row outputs for rows with no banded pair; qdr / dist / dcpa / tcpa / tinconf of every common conflict.
+    ``zone``: (rpz, hpz, dtlookahead) of the detection; ``lat0, lon0``: its origin (default: StateBasedCD.detect's)."""
     n = len(s[0])
     rows = np.arange(n) if rows is None else rows
-    o = statebased.detect_rows(rows, *s, RPZ, HPZ, DTL, with_margins=True)
+    pos_quant = _pos_quant(s, lat0, lon0)
+    o = statebased.detect_rows(rows, *s, *zone, with_margins=True)
     sw, near = o["swconfl"], o["near_conf"]
     gp = set(map(tuple, g["confpairs"].tolist()))
     row_of = {int(r): k for k, r in enumerate(rows)}
@@ -47,8 +62,8 @@ def _check_against_oracle(s, g, rows=None, stats=None, pos_quant=0.5):
     # attributes of the conflicts both sides report (float32 kernel vs float64 oracle; tolerances stated here):
     #   qdr 2e-3 deg (+ 2 pos_quant / dist), dist 1e-5 rel + pos_quant, dcpa 1e-4 rel + 4 pos_quant, tcpa 1e-4 rel + 0.05 s,
     #   tinconf 1e-4 rel + 0.05 s + 1e-2 of the half-width of the horizontal window (sqrt near dcpa = R), banded pairs skipped.
-    #   pos_quant = resolution of the float32 record positions: 0.5 m within ~40 deg of the airspace origin; the antimeridian
-    #   test puts the origin half a world away (x ~ 2e7 m: 2 m steps) on purpose
+    #   pos_quant = resolution of the float32 record positions (_pos_quant): 0.5 m within ~20 deg of the airspace origin; the
+    #   antimeridian test puts the origin half a world away (x ~ 2e7 m: 2 m steps, pos_quant 4 m) on purpose
     err = dict(qdr=0.0, dist=0.0, dcpa=0.0, tcpa=0.0, tinconf=0.0)
     for k, (i, j) in enumerate(map(tuple, g["confpairs"].tolist())):
         if i not in row_of or (i, j) not in op or near[row_of[i], j]:
@@ -70,18 +85,30 @@ def _check_against_oracle(s, g, rows=None, stats=None, pos_quant=0.5):
     return n_exempt, len(op)
 
 
-@pytest.mark.parametrize("n,box", [(2, 0.5), (255, 2.0), (256, 2.0), (257, 2.0), (1000, 4.0), (3000, 6.0), (4096, 40.0)])
-def test_dense_parity(cuda, n, box):
+# zones (rpz, hpz, dtlookahead): the default, a small one and a large one
+ZONES = {"default": (RPZ, HPZ, DTL), "small": (50.0, 15.0, 30.0), "large": (20 * 1852.0, 2000 * 0.3048, 1200.0)}
+DENSE = [(2, 0.5, 52.0, "default"), (255, 2.0, 52.0, "default"), (256, 2.0, 52.0, "default"), (257, 2.0, 52.0, "default"),
+         (1000, 4.0, 52.0, "default"), (3000, 6.0, 52.0, "default"), (4096, 40.0, 52.0, "default"),
+         (2000, 0.08, -45.0, "small"), (2000, 4.0, 0.0, "default"), (2000, 8.0, 70.0, "large"), (1500, 1.5, 85.0, "default"),
+         (1000, 0.6, 89.5, "default"), (2000, 5.0, -45.0, "large")]
+
+
+@pytest.mark.parametrize("n,box,lat0,zone", DENSE, ids=[f"{n}-{b}" if (la, z) == (52.0, "default") else f"{n}-{b}-{la}-{z}"
+                                                        for n, b, la, z in DENSE])
+def test_dense_parity(cuda, n, box, lat0, zone):
+    """Every ordered pair and the default form against the oracle: flight-level traffic at 52 N with the default zone, and
+    with other zones in the southern hemisphere, across the equator, at high latitudes and next to the pole."""
     from bluesky_gym_sasha_b200.cd import StateBasedCD
-    s = synth_airspace(n, box_deg=box, seed=n)
+    zone = ZONES[zone]
+    s = synth_airspace(n, box_deg=box, seed=n, lat0=lat0)
     stats = {}
     for kw in (dict(cull=False, symmetric=False), dict()):             # every ordered pair / the default (culled + symmetric) form
-        g = StateBasedCD(rpz=RPZ, hpz=HPZ, dtlookahead=DTL).detect(*s, **kw)
-        n_exempt, n_conf = _check_against_oracle(s, g, stats=stats)
+        g = StateBasedCD(rpz=zone[0], hpz=zone[1], dtlookahead=zone[2]).detect(*s, **kw)
+        n_exempt, n_conf = _check_against_oracle(s, g, stats=stats, zone=zone)
         assert g["n_conf"] == len(g["confpairs"]) == len(g["tcpa"])
         assert n_exempt <= max(2, n_conf // 200), (n_exempt, n_conf)       # the band must stay a rarity
         assert stats["n_los_exempt"] <= max(2, stats["n_los"] // 100)
-    print(f"N={n}: {n_conf} conflicts ({n_exempt} banded), {stats['n_los']} LoS pairs ({stats['n_los_exempt']} banded); max |error| "
+    print(f"N={n} at {lat0} N, zone {zone}: {n_conf} conflicts ({n_exempt} banded), {stats['n_los']} LoS pairs ({stats['n_los_exempt']} banded); max |error| "
           + ", ".join(f"{k} {stats[k]:.3g}" for k in ("qdr", "dist", "dcpa", "tcpa", "tinconf")))
 
 
@@ -128,7 +155,7 @@ def test_lon_wrap(cuda):
     s = list(synth_airspace(600, box_deg=3.0, seed=5, lat0=10.0, lon0=179.9))
     s[1] = (s[1] + 180.0) % 360.0 - 180.0
     g = StateBasedCD().detect(*s, lon0=0.0)        # origin far away -> the wrap path is taken
-    _check_against_oracle(tuple(s), g, pos_quant=4.0)
+    _check_against_oracle(tuple(s), g, lon0=0.0)
 
 
 def test_row_shards_union(cuda):
