@@ -103,8 +103,8 @@ class TensorTable(C.Structure):
 
 SYMBOLS = ("bsg_abi_version", "bsg_abi_struct_size", "bsg_last_error", "bsg_device_count", "bsg_query_layout", "bsg_create",
            "bsg_destroy", "bsg_bind_state", "bsg_reset", "bsg_step", "bsg_step_host", "bsg_step_host_block", "bsg_step_host_copy", "bsg_step_host_begin", "bsg_step_host_wait", "bsg_host_copy", "bsg_host_widen", "bsg_set_obs_noise", "bsg_get_noise_calls", "bsg_set_noise_calls", "bsg_load_state", "bsg_set_seed", "bsg_set_wind", "bsg_traf_update",
-           "bsg_cd_padded", "bsg_cd_pack", "bsg_cd_order_workspace", "bsg_cd_pack_ordered", "bsg_cd_detect", "bsg_cd_cull_workspace", "bsg_cd_detect_culled", "bsg_cd_detect_peers", "bsg_probe_fp32",
-           "bsg_traf_pack", "bsg_traf_activate", "bsg_traf_workspace", "bsg_traf_substep", "bsg_traf_events_workspace",
+           "bsg_cd_padded", "bsg_cd_pack", "bsg_cd_order_workspace", "bsg_cd_pack_ordered", "bsg_cd_detect", "bsg_cd_cull_workspace", "bsg_cd_detect_culled", "bsg_cd_detect_peers", "bsg_cd_unpermute", "bsg_probe_fp32",
+           "bsg_traf_pack", "bsg_traf_order_workspace", "bsg_traf_pack_ordered", "bsg_traf_activate", "bsg_traf_workspace", "bsg_traf_substep", "bsg_traf_events_workspace",
            "bsg_traf_events_update", "bsg_render")
 
 _lib = None
@@ -161,6 +161,9 @@ def load():
     lib.bsg_render.argtypes = [vp, i32, i32, i32, u32, vp, vp]
     lib.bsg_render.restype = C.c_int
     lib.bsg_traf_pack.argtypes = [C.POINTER(TrafConfig), C.POINTER(TrafTensors), vp, vp]
+    lib.bsg_traf_order_workspace.argtypes = [i64]
+    lib.bsg_traf_order_workspace.restype = i64
+    lib.bsg_traf_pack_ordered.argtypes = [C.POINTER(TrafConfig), C.POINTER(TrafTensors), i32, vp, vp, vp, vp, i64, vp]
     lib.bsg_traf_activate.argtypes = [C.POINTER(TrafConfig), C.POINTER(TrafTensors), vp]
     lib.bsg_traf_substep.argtypes = [C.POINTER(TrafConfig), C.POINTER(TrafTensors), vp, i32, vp, vp, vp, vp, i64, vp, i64, vp]
     lib.bsg_traf_workspace.argtypes = [i64, i64]
@@ -179,12 +182,13 @@ def load():
     lib.bsg_cd_cull_workspace.restype = i64
     lib.bsg_cd_detect_culled.argtypes = [vp, i64, i64, i64, f32, f32, f32, u32, vp, vp, vp, vp, C.POINTER(CdLists), vp, i64, vp]
     lib.bsg_cd_detect_peers.argtypes = [C.POINTER(vp), i32, i32, i64, f32, f32, f32, u32, vp, vp, vp, vp, C.POINTER(CdLists), vp, i64, vp]
+    lib.bsg_cd_unpermute.argtypes = [vp, i64, C.POINTER(CdLists), vp, vp, vp, vp, vp, vp, vp, vp, vp]
     lib.bsg_probe_fp32.argtypes = [i32, C.POINTER(f64)]
     lib.bsg_abi_struct_size.argtypes = [C.c_int]
     lib.bsg_abi_struct_size.restype = C.c_int
     for name in ("bsg_query_layout", "bsg_create", "bsg_bind_state", "bsg_reset", "bsg_step", "bsg_step_host", "bsg_step_host_block", "bsg_step_host_copy",
-                 "bsg_traf_update", "bsg_traf_pack", "bsg_traf_activate", "bsg_traf_substep", "bsg_traf_events_update", "bsg_cd_pack", "bsg_cd_pack_ordered",
-                 "bsg_cd_detect", "bsg_cd_detect_culled", "bsg_cd_detect_peers", "bsg_probe_fp32"):
+                 "bsg_traf_update", "bsg_traf_pack", "bsg_traf_pack_ordered", "bsg_traf_activate", "bsg_traf_substep", "bsg_traf_events_update", "bsg_cd_pack", "bsg_cd_pack_ordered",
+                 "bsg_cd_detect", "bsg_cd_detect_culled", "bsg_cd_detect_peers", "bsg_cd_unpermute", "bsg_probe_fp32"):
         getattr(lib, name).restype = C.c_int
     for which, st in enumerate((Config, Layout, TensorTable, Wind, Perf, AcState, CdLists, TrafConfig, TrafTensors, TrafEvents)):
         if lib.bsg_abi_struct_size(which) != C.sizeof(st):

@@ -15,6 +15,7 @@ import torch
 from . import _lib
 
 NM, FT = 1852.0, 0.3048
+ROW_OUTPUTS = ("nconf_row", "nlos_row", "tcpamax", "inconf")     # per-row outputs of a detection, bsg_cd_unpermute's order
 
 
 def _ptr(t):
@@ -46,19 +47,15 @@ def all_gather_records(rec_local, n_local, group=None, out=None):
     return out
 
 
-def host_lists(out, lists, per_aircraft, perm=None):
+def host_lists(out, lists, per_aircraft):
     """Host form of a detection's pair lists (``detect_packed`` with ``want_pairs``; ``lists``: its ``StateBasedCD.lists``),
     as upstream's detect() returns them: ``confpairs``, ``lospairs`` (up to the lists' capacity, row-major order), the
     host arrays of ``per_aircraft``, ``n_conf``, ``n_los``, ``truncated`` (more pairs found than the lists hold), ``qdr,
-    dist, dcpa, tcpa, tinconf`` per conflict.  ``perm``: record k holds aircraft ``perm[k]`` (``pack_ordered``).
-    Synchronises the device."""
+    dist, dcpa, tcpa, tinconf`` per conflict.  Synchronises the device."""
     torch.cuda.synchronize(out["npairs"].device)
     n_conf, n_los = (int(v) for v in out["npairs"].cpu())
     k, kl = min(n_conf, lists.conf_cap), min(n_los, lists.los_cap)
     pairs, lospairs, attr = out["pairs"][:k], out["lospairs"][:kl], out["attr"][:k]
-    if perm is not None:
-        pairs = perm[pairs.long()].to(torch.int32)
-        lospairs = perm[lospairs.long()].to(torch.int32)
     # upstream's order: row-major np.where (own index, then intruder index).  Keys are unique, so one sort of the
     # combined 64-bit key on the device orders a list
     o = torch.argsort(pairs[:, 0].long() * (1 << 32) + pairs[:, 1].long())
@@ -218,25 +215,30 @@ class StateBasedCD:
             lon0 = float(lon_d[0])
         span = float((((lon_d - lon0) + 180.0) % 360.0 - 180.0).abs().max())
         cull = cull and span < 90.0                       # (airspaces across the antimeridian: plain form)
-        perm = None
         if cull:
             rec, n, perm = self.pack_ordered(lat_d, lon_d, trk, gs, alt, vs, lat0, lon0)
-            perm = perm.long()
         else:
             rec, n = self.pack(lat_d, lon_d, trk, gs, alt, vs, lat0, lon0)
         out = self.detect_packed(rec, n, lon_wrap=span >= 90.0, cull=cull, symmetric=symmetric and span < 90.0)
-        inconf, tcpamax = out["inconf"], out["tcpamax"]
-        nconf_row, nlos_row = out["nconf_row"], out["nlos_row"]
-        if perm is not None:                              # back to the caller's aircraft order
-            def unperm(x):
-                y = torch.empty_like(x)
-                y[perm] = x
-                return y
-            inconf, tcpamax, nconf_row, nlos_row = (unperm(x) for x in (inconf, tcpamax, nconf_row, nlos_row))
-        return host_lists(out, self.lists, dict(inconf=inconf.cpu().numpy().astype(bool),
-                                                tcpamax=tcpamax.cpu().numpy().astype(np.float64),
-                                                nconf_row=nconf_row.cpu().numpy().astype(np.int64),
-                                                nlos_row=nlos_row.cpu().numpy().astype(np.int64)), perm)
+        if cull:                                          # back to the caller's aircraft order
+            out = self.unpermute(perm, n, out)
+        return host_lists(out, self.lists, dict(inconf=out["inconf"].cpu().numpy().astype(bool),
+                                                tcpamax=out["tcpamax"].cpu().numpy().astype(np.float64),
+                                                nconf_row=out["nconf_row"].cpu().numpy().astype(np.int64),
+                                                nlos_row=out["nlos_row"].cpu().numpy().astype(np.int64)))
+
+    def unpermute(self, perm, n, out, per_row=None):
+        """Outputs of ``detect_packed`` on records in the order ``perm`` (record k = aircraft ``perm[k]``) in aircraft
+        order (bsg_cd_unpermute, asynchronous): the pair lists of ``self.lists`` are rewritten in place, the per-row outputs
+        scattered into ``per_row`` (dict of ``nconf_row, nlos_row, tcpamax, inconf`` tensors of at least n rows; default:
+        buffers of this object).  Returns ``out`` with the per-row entries replaced by the first n rows of those."""
+        if per_row is None:
+            per_row = {k: self._get("unperm_" + k, (max(n, 1),), out[k].dtype) for k in ROW_OUTPUTS}
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.bsg_cd_unpermute(_ptr(perm), n, C.byref(self.lists), *[_ptr(out[k]) for k in ROW_OUTPUTS],
+                                                 *[_ptr(per_row[k]) for k in ROW_OUTPUTS], self._stream()))
+        self.gpu_launches += 1
+        return dict(out, **{k: per_row[k][:n] for k in ROW_OUTPUTS})
 
     # ---------------------------------------------------------------- multi-GPU: rows sharded over ranks
     def detect_sharded(self, rec_local, n_local, group=None, lon_wrap=False, want_pairs=False, cull=False):

@@ -44,11 +44,27 @@ __global__ void order_init_kernel(OrderWork* w) {
     if (i == 0) { w->box[0] = w->box[2] = 0x7fffffffffffffffLL; w->box[1] = w->box[3] = -0x7fffffffffffffffLL - 1; }
 }
 
-__global__ void __launch_bounds__(256) order_bbox_kernel(const double* __restrict__ lat, const double* __restrict__ lon, long long n,
-                                                         double lon0, OrderWork* w) {
+// where the order kernels read an aircraft's position: the float64 SoA arrays of bsg_cd_pack_ordered, or the traffic
+// state of bsg_traf_pack_ordered, whose dead slots (inert records) stay out of the bounding box
+struct SoaPos {
+    const double *lat, *lon;
+    __device__ __forceinline__ bool in_box(long long) const { return true; }
+    __device__ __forceinline__ double2 operator()(long long i) const { return make_double2(lat[i], lon[i]); }
+};
+struct TrafPos {
+    const double2* pos;
+    const uint32_t* flags;
+    __device__ __forceinline__ bool in_box(long long i) const { return (flags[i] & BSG_TF_ALIVE) != 0; }
+    __device__ __forceinline__ double2 operator()(long long i) const { return pos[i]; }
+};
+
+template <typename Pos>
+__global__ void __launch_bounds__(256) order_bbox_kernel(const Pos pos, long long n, double lon0, OrderWork* w) {
     double a0 = 1e300, a1 = -1e300, o0 = 1e300, o1 = -1e300;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
-        const double la = lat[i], dl = dlon_of(lon[i], lon0);
+        if (!pos.in_box(i)) continue;
+        const double2 p = pos(i);
+        const double la = p.x, dl = dlon_of(p.y, lon0);
         a0 = fmin(a0, la); a1 = fmax(a1, la); o0 = fmin(o0, dl); o1 = fmax(o1, dl);
     }
     for (int o = 16; o > 0; o >>= 1) {
@@ -76,15 +92,16 @@ __device__ __forceinline__ void order_grid(const OrderWork* w, long long n, doub
     sy = (double)ny / h * (1.0 - 1e-12); sx = (double)nx / fmax(o1 - o0, 1e-9) * (1.0 - 1e-12);
 }
 
-__global__ void __launch_bounds__(256) order_cell_kernel(const double* __restrict__ lat, const double* __restrict__ lon, long long n,
-                                                         double lon0, OrderWork* w, int* __restrict__ cell) {
+template <typename Pos>
+__global__ void __launch_bounds__(256) order_cell_kernel(const Pos pos, long long n, double lon0, OrderWork* w, int* __restrict__ cell) {
     double la0, o0, sy, sx;
     int ny, nx;
     order_grid(w, n, la0, o0, sy, sx, ny, nx);
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i == 0) { w->grid[0] = ny; w->grid[1] = nx; w->grid[2] = ny * nx; }
     if (i >= n) return;
-    int iy = (int)((lat[i] - la0) * sy), ix = (int)((dlon_of(lon[i], lon0) - o0) * sx);
+    const double2 p = pos(i);
+    int iy = (int)((p.x - la0) * sy), ix = (int)((dlon_of(p.y, lon0) - o0) * sx);
     iy = min(max(iy, 0), ny - 1); ix = min(max(ix, 0), nx - 1);
     if (iy & 1) ix = nx - 1 - ix;                      // alternate strips run the other way
     const int c = iy * nx + ix;
@@ -123,6 +140,58 @@ __global__ void __launch_bounds__(256) order_scatter_kernel(long long n, OrderWo
     perm[w->offs[c] + atomicAdd(&w->hist[c], 1)] = (int32_t)i;
 }
 
+// a detection on ordered records -> aircraft order: pair list rows (the first min(npairs, cap), count read here) are
+// rewritten in place through perm, per-row outputs scattered, out[perm[k]] = in[k].  One grid-stride range over the conflict
+// rows, then the LoS rows, then the aircraft, so that each thread has one short chain of dependent loads: O(pairs + n).
+struct UnpermArgs {
+    const int32_t* perm;
+    long long n;
+    int2 *conf, *los;
+    long long conf_cap, los_cap;
+    const unsigned long long* npairs;
+    const uint32_t *nconf_in, *nlos_in;
+    const float* tcpamax_in;
+    const uint8_t* inconf_in;
+    uint32_t *nconf_out, *nlos_out;
+    float* tcpamax_out;
+    uint8_t* inconf_out;
+};
+
+__global__ void __launch_bounds__(256) cd_unpermute_kernel(const UnpermArgs a) {
+    const long long t0 = (long long)blockIdx.x * blockDim.x + threadIdx.x, stride = (long long)gridDim.x * blockDim.x;
+    const int32_t* __restrict__ perm = a.perm;
+    const long long mc = a.conf ? (long long)min(a.npairs[0], (unsigned long long)a.conf_cap) : 0;
+    const long long ml = a.los ? (long long)min(a.npairs[1], (unsigned long long)a.los_cap) : 0;
+    for (long long t = t0; t < mc + ml + a.n; t += stride) {
+        if (t < mc + ml) {
+            int2* __restrict__ row = t < mc ? a.conf + t : a.los + (t - mc);
+            const int2 p = *row;
+            *row = make_int2(perm[p.x], perm[p.y]);
+        } else {
+            const long long k = t - mc - ml;
+            const int32_t j = perm[k];
+            if (a.nconf_out) a.nconf_out[j] = a.nconf_in[k];
+            if (a.nlos_out) a.nlos_out[j] = a.nlos_in[k];
+            if (a.tcpamax_out) a.tcpamax_out[j] = a.tcpamax_in[k];
+            if (a.inconf_out) a.inconf_out[j] = a.inconf_in[k];
+        }
+    }
+}
+
+// the order of n aircraft into perm: bounding box, cells, scan, scatter (five launches)
+template <typename Pos>
+static int order_launch(const Pos pos, long long n, double lon0, int32_t* perm, void* d_work, cudaStream_t st) {
+    OrderWork* w = (OrderWork*)d_work;
+    int* cell = (int*)((char*)d_work + sizeof(OrderWork));
+    const int blocks = (int)((n + 255) / 256);
+    order_init_kernel<<<kOrderMaxCells / 256, 256, 0, st>>>(w);
+    order_bbox_kernel<<<blocks < 592 ? blocks : 592, 256, 0, st>>>(pos, n, lon0, w);
+    order_cell_kernel<<<blocks, 256, 0, st>>>(pos, n, lon0, w, cell);
+    order_scan_kernel<<<1, 1024, 0, st>>>(w);
+    order_scatter_kernel<<<blocks, 256, 0, st>>>(n, w, cell, perm);
+    return bsg_cuda_check(cudaGetLastError(), "spatial order launch");
+}
+
 }  // namespace bsg
 
 using namespace bsg;
@@ -143,15 +212,48 @@ extern "C" int bsg_cd_pack_ordered(const double* d_lat, const double* d_lon, con
     if (!d_work || work_bytes < bsg_cd_order_workspace(n)) return bsg_fail(BSG_EINVAL, "bsg_cd_pack_ordered: workspace too small");
     if ((uintptr_t)d_work % 8) return bsg_fail(BSG_EINVAL, "bsg_cd_pack_ordered: workspace must be 8-byte aligned");
     cudaStream_t st = (cudaStream_t)stream;
-    OrderWork* w = (OrderWork*)d_work;
-    int* cell = (int*)((char*)d_work + sizeof(OrderWork));
-    const int blocks = (int)((n + 255) / 256);
-    order_init_kernel<<<kOrderMaxCells / 256, 256, 0, st>>>(w);
-    order_bbox_kernel<<<blocks < 592 ? blocks : 592, 256, 0, st>>>(d_lat, d_lon, n, lon0, w);
-    order_cell_kernel<<<blocks, 256, 0, st>>>(d_lat, d_lon, n, lon0, w, cell);
-    order_scan_kernel<<<1, 1024, 0, st>>>(w);
-    order_scatter_kernel<<<blocks, 256, 0, st>>>(n, w, cell, d_perm);
-    int rc = bsg_cuda_check(cudaGetLastError(), "bsg_cd_pack_ordered launch");
+    int rc = order_launch(SoaPos{d_lat, d_lon}, n, lon0, d_perm, d_work, st);
     if (rc != BSG_OK) return rc;
     return bsg_cd_pack_launch(d_lat, d_lon, d_trk, d_gs, d_alt, d_vs, d_perm, n, lat0, lon0, d_rec, st);
+}
+
+// (traf_airspace.cu: bsg_traf_pack_ordered; the caller has validated the arguments and the workspace)
+int bsg_traf_order_launch(const double2* pos, const uint32_t* flags, int64_t n, double lon0, int32_t* d_perm, void* d_work,
+                          cudaStream_t st) {
+    return order_launch(TrafPos{pos, flags}, n, lon0, d_perm, d_work, st);
+}
+
+extern "C" int bsg_cd_unpermute(const int32_t* d_perm, int64_t n, const bsg_cd_lists* lists, const uint32_t* d_nconf_in,
+                                const uint32_t* d_nlos_in, const float* d_tcpamax_in, const uint8_t* d_inconf_in,
+                                uint32_t* d_nconf_out, uint32_t* d_nlos_out, float* d_tcpamax_out, uint8_t* d_inconf_out,
+                                void* stream) {
+    if (n < 0 || n > 0x7fffff00LL) return bsg_fail(BSG_EINVAL, "bsg_cd_unpermute: n must be in [0, 2^31 - 256]");
+    if (n > 0 && !d_perm) return bsg_fail(BSG_EINVAL, "bsg_cd_unpermute: null d_perm");
+    if ((!d_nconf_in != !d_nconf_out) || (!d_nlos_in != !d_nlos_out) || (!d_tcpamax_in != !d_tcpamax_out) ||
+        (!d_inconf_in != !d_inconf_out))
+        return bsg_fail(BSG_EINVAL, "bsg_cd_unpermute: a per-row output needs both its input and its output pointer");
+    if ((d_nconf_in && (const void*)d_nconf_in == (const void*)d_nconf_out) ||
+        (d_nlos_in && (const void*)d_nlos_in == (const void*)d_nlos_out) ||
+        (d_tcpamax_in && (const void*)d_tcpamax_in == (const void*)d_tcpamax_out) ||
+        (d_inconf_in && (const void*)d_inconf_in == (const void*)d_inconf_out))
+        return bsg_fail(BSG_EINVAL, "bsg_cd_unpermute: per-row input and output must be distinct (a scatter cannot run in place)");
+    UnpermArgs a{};
+    a.perm = d_perm; a.n = n;
+    if (lists) {
+        if (lists->conf_cap < 0 || lists->los_cap < 0) return bsg_fail(BSG_EINVAL, "bsg_cd_unpermute: negative list capacities");
+        if ((lists->d_conf_pairs || lists->d_los_pairs) && !lists->d_npairs)
+            return bsg_fail(BSG_EINVAL, "bsg_cd_unpermute: pair lists need d_npairs");
+        a.conf = lists->conf_cap > 0 ? (int2*)lists->d_conf_pairs : nullptr;
+        a.los = lists->los_cap > 0 ? (int2*)lists->d_los_pairs : nullptr;
+        a.conf_cap = lists->conf_cap; a.los_cap = lists->los_cap; a.npairs = lists->d_npairs;
+    }
+    if (n == 0) a.conf = a.los = nullptr;               // no records, no pairs
+    a.nconf_in = d_nconf_in; a.nlos_in = d_nlos_in; a.tcpamax_in = d_tcpamax_in; a.inconf_in = d_inconf_in;
+    a.nconf_out = d_nconf_out; a.nlos_out = d_nlos_out; a.tcpamax_out = d_tcpamax_out; a.inconf_out = d_inconf_out;
+    // threads: one per aircraft and list row (at most), up to 8 blocks per SM
+    const long long work = n + (a.conf ? a.conf_cap : 0) + (a.los ? a.los_cap : 0);
+    if (work == 0) return BSG_OK;
+    const long long blocks = (work + 255) / 256;
+    cd_unpermute_kernel<<<(unsigned)(blocks < 1184 ? blocks : 1184), 256, 0, (cudaStream_t)stream>>>(a);
+    return bsg_cuda_check(cudaGetLastError(), "bsg_cd_unpermute launch");
 }

@@ -128,11 +128,10 @@ __device__ __forceinline__ void traf_store(const Ac& a, const TrafAc& x, const T
     P.flags[i] = x.f;
 }
 
-__global__ void traf_pack_kernel(const TrafParams P, float* __restrict__ rec, const long long n_pad) {
-    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n_pad) return;
-    float f[BSG_CD_REC_FIELDS];
-    cd_rec_inert(f);                                                        // padding / dead slots
+// CD record of aircraft i (inert for padding and dead slots).  The one record computation of both packs: a reordered
+// record is bit for bit the aircraft-order record.
+__device__ __forceinline__ void traf_record(const TrafParams& P, const long long i, float (&f)[BSG_CD_REC_FIELDS]) {
+    cd_rec_inert(f);
     if (i < P.n && (P.flags[i] & BSG_TF_ALIVE)) {
         const double2 p = P.pos[i];
         const float4 k = P.kin[i];
@@ -141,7 +140,27 @@ __global__ void traf_pack_kernel(const TrafParams P, float* __restrict__ rec, co
         sincosf(k.z * kDeg2Rad, &sh, &ch);
         f[FU] = k.y * sh; f[FV] = k.y * ch; f[FALT] = k.x; f[FVS] = k.w;
     }
+}
+
+__global__ void traf_pack_kernel(const TrafParams P, float* __restrict__ rec, const long long n_pad) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_pad) return;
+    float f[BSG_CD_REC_FIELDS];
+    traf_record(P, i, f);
     cd_rec_store(rec, i, f);
+}
+
+// gather: record slot k <- aircraft perm[k] (slots past n: inert), and the same record into aircraft order when rec != NULL
+__global__ void __launch_bounds__(256) traf_pack_ordered_kernel(const TrafParams P, const int32_t* __restrict__ perm,
+                                                                float* __restrict__ rec_ordered, float* __restrict__ rec,
+                                                                const long long n_pad) {
+    const long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n_pad) return;
+    const long long i = k < P.n ? (long long)perm[k] : k;
+    float f[BSG_CD_REC_FIELDS];
+    traf_record(P, i, f);
+    cd_rec_store(rec_ordered, k, f);
+    if (rec) cd_rec_store(rec, i, f);
 }
 
 __global__ void traf_activate_kernel(const TrafParams P) {
@@ -492,6 +511,35 @@ extern "C" int bsg_traf_pack(const bsg_traf_config* cfg, const bsg_traf_tensors*
     if (n_pad == 0) return BSG_OK;
     traf_pack_kernel<<<(unsigned)(n_pad / 256), 256, 0, (cudaStream_t)stream>>>(P, d_rec, n_pad);
     return bsg_cuda_check(cudaGetLastError(), "bsg_traf_pack launch");
+}
+
+// (cd_order.cu)
+int bsg_traf_order_launch(const double2* pos, const uint32_t* flags, int64_t n, double lon0, int32_t* d_perm, void* d_work,
+                          cudaStream_t st);
+
+extern "C" int64_t bsg_traf_order_workspace(int64_t n) { return bsg_cd_order_workspace(n); }
+
+extern "C" int bsg_traf_pack_ordered(const bsg_traf_config* cfg, const bsg_traf_tensors* t, int32_t reorder, int32_t* d_perm,
+                                     float* d_rec_ordered, float* d_rec, void* d_work, int64_t work_bytes, void* stream) {
+    TrafParams P;
+    int rc = traf_params(P, cfg, t, "bsg_traf_pack_ordered");
+    if (rc != BSG_OK) return rc;
+    if (P.row0 != 0) return bsg_fail(BSG_EINVAL, "bsg_traf_pack_ordered: not for an airspace sharded over GPUs (row0 != 0)");
+    if (!d_perm || !d_rec_ordered) return bsg_fail(BSG_EINVAL, "bsg_traf_pack_ordered: null d_perm or d_rec_ordered");
+    if (reorder) {
+        if (!d_work || work_bytes < bsg_traf_order_workspace(P.n))
+            return bsg_fail(BSG_EINVAL, "bsg_traf_pack_ordered: workspace too small (bsg_traf_order_workspace)");
+        if ((uintptr_t)d_work % 8) return bsg_fail(BSG_EINVAL, "bsg_traf_pack_ordered: workspace must be 8-byte aligned");
+    }
+    const long long n_pad = bsg_cd_padded(P.n);
+    if (n_pad == 0) return BSG_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (reorder) {
+        rc = bsg_traf_order_launch(P.pos, P.flags, P.n, P.lon0, d_perm, d_work, st);
+        if (rc != BSG_OK) return rc;
+    }
+    traf_pack_ordered_kernel<<<(unsigned)(n_pad / 256), 256, 0, st>>>(P, d_perm, d_rec_ordered, d_rec, n_pad);
+    return bsg_cuda_check(cudaGetLastError(), "bsg_traf_pack_ordered launch");
 }
 
 extern "C" int bsg_traf_activate(const bsg_traf_config* cfg, const bsg_traf_tensors* t, void* stream) {

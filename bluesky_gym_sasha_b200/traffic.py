@@ -5,6 +5,8 @@ Interface mirrored: the handful of ``bs.traf`` / ``bs.stack`` calls a BlueSky sc
 select commands, ``RESO MVP`` / ``RESO OFF`` (``reso=``; the reference's own line is ``reso off``, merge_env.py:157),
 ``RESOOFF acid``, ``bs.sim.step()`` (``step``) -- with the state arrays ``lat, lon, alt, tas, hdg, vs, ...`` as properties.
 Per substep: ``bsg_traf_pack`` -> ``bsg_cd_detect[_culled]`` with pair lists (K2) -> ``bsg_traf_substep`` (include/bsg.h).  Restated for checking in oracle/traffic_ext.py.  No CPU fallback.
+With ``reorder_dt`` the culled detection runs on records in a spatial order kept on the device (``bsg_traf_pack_ordered``,
+``bsg_cd_unpermute``): the same results, without relying on the aircraft being created in a spatially coherent order.
 With ``events=True`` each detection also feeds ``bsg_traf_events_update``: the conflict / LoS event counts and logs of
 upstream's ConflictDetection.update (``conflict_counts``, ``conflict_log``; restated in oracle/conflict_log.py).
 """
@@ -97,7 +99,7 @@ class AirspaceTraffic:
 
     def __init__(self, n_max, device=0, simdt=1.0, rpz=5.0 * NM, hpz=1000.0 * FT, dtlookahead=300.0, reso=None, reso_mode=0,
                  resofach=1.01, resofacv=1.01, perf=None, max_wpts=8, lat0=52.0, lon0=4.0, cull=True, symmetric=True,
-                 pair_capacity=None, fms_dt=10.5, group=None, events=False, event_capacity=None):
+                 pair_capacity=None, fms_dt=10.5, group=None, events=False, event_capacity=None, reorder_dt=None):
         """``group``: a ``torch.distributed`` process group (``True`` = the default group) over which ONE airspace is sharded,
         one rank per GPU (SURVEY 8e): every rank owns the kinematics of up to ``n_max`` aircraft (its block); per substep the
         ranks all-gather their CD records (32 B per aircraft over NVLink), each detects the conflicts of its own rows against
@@ -107,9 +109,24 @@ class AirspaceTraffic:
         ConflictDetection.update (confpairs_all / lospairs_all) on the device (bsg_traf_events_update), read with
         ``conflict_counts()`` and ``conflict_log()``.  ``event_capacity``: rows of each event log (default 8 x n_max); the
         totals stay exact when a log is full.  Not with ``group``: on a row-sharded rank the two orders of a pair sit on
-        different GPUs, so counting unordered pairs would need an exchange of the pair lists."""
-        if events and group is not None and group is not False:
+        different GPUs, so counting unordered pairs would need an exchange of the pair lists.
+
+        ``reorder_dt``: simulated seconds between fresh spatial orders of the CD records.  The culled detection only skips
+        work when consecutive records are close in space; by default the records follow the aircraft index, so that holds
+        only for aircraft created in a spatially sorted order, and less so the longer they fly.  With ``reorder_dt`` the
+        detection runs on records in a grid order recomputed on the device every ``max(1, reorder_dt // simdt)`` substeps
+        (and at the first detection after ``create()``), and its outputs are mapped back to aircraft order: every result
+        is identical.  ``record_order`` is the current order.  Needs ``cull=True``; not with ``group``."""
+        sharded = group is not None and group is not False
+        if events and sharded:
             raise ValueError("events=True is not available for an airspace sharded over a process group")
+        if reorder_dt is not None:
+            if sharded:
+                raise ValueError("reorder_dt is not available for an airspace sharded over a process group")
+            if not cull:
+                raise ValueError("reorder_dt orders the records for the culled detection: it needs cull=True")
+            if not reorder_dt > 0:
+                raise ValueError("reorder_dt must be > 0")
         if not torch.cuda.is_available():
             raise _lib.BsgError("AirspaceTraffic needs a CUDA device: there is no CPU fallback")
         if reso not in (None, "OFF", "MVP"):
@@ -139,11 +156,19 @@ class AirspaceTraffic:
                       rt_pos=z(n, W, 2, dt=torch.float64), rt_con=z(n, W, 4), rt_dir=z(n, W),
                       counters=z(_lib.TRAF_CTR_COUNT, dt=torch.int32))
         self.tt = _lib.TrafTensors(**{k: _ptr(v) for k, v in self.t.items()})
-        sharded = group is not None and group is not False
         # (sharded: records this rank never packs, beyond its aircraft count, stay inert)
         self.rec = cd_records(n, dev, inert=sharded)
         self.work = torch.zeros(int(self.lib.bsg_traf_workspace(n, cap)), dtype=torch.uint8, device=dev)      # (zeroed once)
         self.last = None                    # device outputs of the last substep's detection
+        self.reorder_freq = None if reorder_dt is None else max(1, int(float(reorder_dt) // self.simdt))
+        if self.reorder_freq:
+            # records in spatial order (record k = aircraft perm[k]) and the detection's per-aircraft outputs mapped back
+            self.rec_ordered = cd_records(n, dev)
+            self.perm = torch.zeros(max(n, 1), dtype=torch.int32, device=dev)
+            self.order_work = torch.empty(int(self.lib.bsg_traf_order_workspace(n)), dtype=torch.uint8, device=dev)
+            self.per_row = dict(nconf_row=z(n, dt=torch.int32), nlos_row=z(n, dt=torch.int32), tcpamax=z(n),
+                                inconf=z(n, dt=torch.uint8))
+            self.order_n = -1               # aircraft count of the current order (-1: none yet)
         self.gpu_launches = 0
         self.events = bool(events)
         if self.events:
@@ -207,6 +232,9 @@ class AirspaceTraffic:
         t["partners"][s] = -1
         self.n += k
         self.cfg.n = self.n
+        # bsg_traf_substep lays its workspace out by n: the per-aircraft counters it needs zero now reach into what were
+        # other arrays
+        self.work.zero_()
         return range(s.start, s.stop)
 
     # ------------------------------------------------------------------ ADDWPT x n + LNAV / VNAV ON
@@ -277,8 +305,10 @@ class AirspaceTraffic:
                 pairs = attr = npairs = nall = None
                 rec = self.rec
                 if detect:
-                    _lib.check(self.lib.bsg_traf_pack(C.byref(self.cfg), C.byref(self.tt), _ptr(self.rec), st))
-                    if self.world > 1:
+                    if self.reorder_freq:
+                        out = self._detect_ordered(n, st)
+                    elif self.world > 1:
+                        _lib.check(self.lib.bsg_traf_pack(C.byref(self.cfg), C.byref(self.tt), _ptr(self.rec), st))
                         import torch.distributed as dist
                         rec = self.allrec = all_gather_records(self.rec, self.per, self.group, self.allrec)
                         out = cd.detect_packed(rec, self.per * self.world, row0=self.row0, n_rows=n, want_pairs=True, cull=self.cull)
@@ -287,6 +317,7 @@ class AirspaceTraffic:
                             dist.all_reduce(self.nconf_all, group=self.group)
                             nall = self.nconf_all
                     else:
+                        _lib.check(self.lib.bsg_traf_pack(C.byref(self.cfg), C.byref(self.tt), _ptr(self.rec), st))
                         out = cd.detect_packed(rec, n, want_pairs=True, cull=self.cull, symmetric=self.symmetric)
                     self.last = out
                     self.gpu_launches += 1
@@ -300,6 +331,22 @@ class AirspaceTraffic:
                                                      cd.pair_capacity if pairs is not None else 0,
                                                      _ptr(self.work), self.work.numel(), st))
                 self.gpu_launches += 1
+
+    def _detect_ordered(self, n, st):
+        """Pack (aircraft order into self.rec, spatial order into self.rec_ordered; a fresh order at the cadence and after
+        the aircraft count changed), detect on the ordered records, map the outputs back to aircraft order."""
+        reorder = self.order_n != n or self.nstep % self.reorder_freq == 0
+        _lib.check(self.lib.bsg_traf_pack_ordered(C.byref(self.cfg), C.byref(self.tt), int(reorder), _ptr(self.perm),
+                                                  _ptr(self.rec_ordered), _ptr(self.rec), _ptr(self.order_work),
+                                                  self.order_work.numel(), st))
+        self.order_n = n
+        self.gpu_launches += 5 if reorder else 0        # (the pack itself is counted with the detection)
+        out = self.cd.detect_packed(self.rec_ordered, n, want_pairs=True, cull=True, symmetric=self.symmetric)
+        self.gpu_launches += 1                          # bsg_cd_unpermute
+        return self.cd.unpermute(self.perm, n, out, self.per_row)
+
+    record_order = property(lambda s: s.perm[:s.n] if s.reorder_freq else None,
+                            doc="With ``reorder_dt``: record k of the detection's input holds aircraft ``record_order[k]``.")
 
     def _track_events(self, st):
         """bsg_traf_events_update on this detection's lists, then the sets swap roles."""

@@ -313,6 +313,15 @@ typedef struct bsg_cd_lists {
     unsigned long long *d_npairs;       /* [2]: conflicts found, LoS pairs found (required with any list)   */
 } bsg_cd_lists;
 
+/* Maps the outputs of a detection on reordered records (record k = aircraft d_perm[k], d_perm a permutation of [0, n))
+ * back to aircraft order, on the device.  The rows of both pair lists of `lists` -- the first min(npairs, cap) of each,
+ * npairs read on the device (no host synchronisation) -- are rewritten in place, (a, b) -> (d_perm[a], d_perm[b]); rows
+ * past them are untouched, the attributes stay as they are.  Per-row outputs are scattered, out[d_perm[k]] = in[k], k < n;
+ * each in / out pair may be NULL (both), and must not alias.  `lists` may be NULL.  One launch, O(pairs + n). */
+int bsg_cd_unpermute(const int32_t *d_perm, int64_t n, const bsg_cd_lists *lists, const uint32_t *d_nconf_in,
+                     const uint32_t *d_nlos_in, const float *d_tcpamax_in, const uint8_t *d_inconf_in,
+                     uint32_t *d_nconf_out, uint32_t *d_nlos_out, float *d_tcpamax_out, uint8_t *d_inconf_out, void *stream);
+
 /* Rows [row0, row0+n_rows) of d_rec against all n_all aircraft (row sharding for multi-GPU).
  * Outputs (caller-owned, device): per-row nconf / nlos counts and tcpamax, inconf flags, and the pair lists
  * (`lists` may be NULL).  Any output pointer except d_nconf_row may be NULL.
@@ -398,13 +407,25 @@ typedef struct bsg_traf_tensors {
 } bsg_traf_tensors;
 /* Traffic state -> CD records of bsg_cd_detect (trk = hdg, gs = tas: no wind); d_rec holds bsg_cd_padded(n) records. */
 int bsg_traf_pack(const bsg_traf_config *cfg, const bsg_traf_tensors *t, float *d_rec, void *stream);
+/* bsg_traf_pack with the records in a spatial order, for bsg_cd_detect_culled on an airspace whose index order is not
+ * spatially coherent (created in any order, or flown for a long time).  reorder != 0: a fresh order of the n aircraft is
+ * computed from their current positions into d_perm [n] (bsg_cd_pack_ordered's grid; dead slots stay out of the bounding
+ * box); reorder == 0: the d_perm given is reused.  Record k of d_rec_ordered (bsg_cd_padded(n) records) is then aircraft
+ * d_perm[k]'s record, bit for bit the one bsg_traf_pack writes, and padding is inert.  d_rec != NULL: the same launch also
+ * writes the aircraft-order records of bsg_traf_pack (what bsg_traf_substep and bsg_traf_events_update read).  Map the
+ * detection's outputs back with bsg_cd_unpermute.  d_work (needed with reorder != 0): 8-byte aligned device scratch of
+ * bsg_traf_order_workspace(n) bytes.  Not for a sharded airspace (cfg->row0 must be 0).  Launches: 5 + 1 with reorder,
+ * else 1. */
+int64_t bsg_traf_order_workspace(int64_t n);
+int bsg_traf_pack_ordered(const bsg_traf_config *cfg, const bsg_traf_tensors *t, int32_t reorder, int32_t *d_perm,
+                          float *d_rec_ordered, float *d_rec, void *d_work, int64_t work_bytes, void *stream);
 /* Route.direct(first waypoint) + ComputeVNAV for every aircraft flagged BSG_TF_ACTIVATE (after the route tables changed). */
 int bsg_traf_activate(const bsg_traf_config *cfg, const bsg_traf_tensors *t, void *stream);
 /* One simulator substep.  d_rec: the records bsg_traf_pack made of the state BEFORE this substep (what the detection saw);
  * d_conf_pairs [conf_cap][2], d_conf_attr [conf_cap][BSG_CD_ATTR_COUNT], d_npairs: the conflict list of that detection
  * exactly as bsg_cd_detect[_culled] wrote it (bsg_cd_lists: any order); all may be NULL with reso == 0.
  * d_work: device scratch of at least bsg_traf_workspace(n, conf_cap) bytes whose first n int32 are ZERO on entry (zero it
- * once after allocation: every call leaves them zero again).  fms_ready: the FMS timer fires in this substep (sim step
+ * after allocation and whenever n changes: every call leaves them zero again).  fms_ready: the FMS timer fires in this substep (sim step
  * count % (10.5 // simdt) == 0).  Airspace sharded over GPUs (cfg->row0 = this block's first global index; SURVEY 8e: a rank
  * owns the kinematics of its block): d_rec holds the records of the WHOLE airspace (every rank's bsg_traf_pack output, all-gathered),
  * the conflict list that of bsg_cd_detect*(row0, n_rows = this block) with global indices, and d_nconf_all the number of
